@@ -363,11 +363,11 @@ def run_ours(args):
             if from_host:
                 host_eloc.copy_(eloc, non_blocking=True)  # D2H of the step's result
                 st = st.result()
-            return st
+            return eloc, psi0, st
 
         def timed(n_steps: int, from_host: bool):
             total_ms = 0.0
-            st = None
+            eloc = psi0 = st = None
             for _ in range(n_steps):
                 flush.fill_(1)  # write > L2 (126 MB) between timed steps
                 torch.cuda.synchronize()
@@ -375,32 +375,36 @@ def run_ours(args):
                     dist.barrier()
                 s, t = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 s.record()
-                st = step(from_host)
+                eloc, psi0, st = step(from_host)
                 t.record()
                 torch.cuda.synchronize()
                 total_ms += s.elapsed_time(t)
             tt = torch.tensor([total_ms], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(tt, op=dist.ReduceOp.MAX)
-            return float(tt.item()), st
+            return float(tt.item()), (eloc, psi0, st)
 
         for _ in range(max(warmup, 4)):  # eager steps, then the capture, then replays
             step(False)
         torch.cuda.synchronize()
         l0 = _lib.launch_count()
-        total_ms, st = timed(steps, False)
+        total_ms, (eloc, psi0, st) = timed(steps, False)
         launches = _lib.launch_count() - l0
+        stats = st.result()
+        last = None
+        if args.dump_outputs:  # copied now: the steps that follow reuse the step's output buffers
+            last = {"eloc": eloc.cpu().numpy(), "psi0": psi0.cpu().numpy(), "stats": stats}
         if step_obj.graph is not None:  # replays do not pass through the library's launch counter: count one eager step
             l0 = _lib.launch_count()
             step_obj._body()
             launches = (_lib.launch_count() - l0) * steps
         out = {"n_total": n_total, "ms_per_step": total_ms / steps, "value": n_total / (total_ms / steps * 1e-3), "launches": int(launches),
-               "stats": st.result(), "cplx": cplx, "graph": step_obj.graph is not None, "why_eager": step_obj.why_eager}
+               "stats": stats, "last_step": last, "cplx": cplx, "graph": step_obj.graph is not None, "why_eager": step_obj.why_eager}
         if want_e2e:
             for _ in range(2):  # the end-to-end path has first-use costs of its own (pinned copies both ways)
                 step(True)
             torch.cuda.synchronize()
-            e2e_ms, st2 = timed(steps, True)
+            e2e_ms, (_, _, st2) = timed(steps, True)
             out["e2e"] = {"value": n_total / (e2e_ms / steps * 1e-3), "unit": UNIT, "h2d_bytes_per_step": int(n_total * (8 + d_psi.element_size())),
                           "d2h_bytes_per_step": int(n_total * d_psi.element_size() + 56 * world), "ms_per_step": e2e_ms / steps}
             out["mean_e2e"] = st2["mean"]
@@ -446,11 +450,13 @@ def run_ours(args):
         sampler.start()
     main = measure(keys_np, psi_np, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main["last_step"], rank, world)
     n_total = main["n_total"]
 
-    # variants (shorter runs of the same step): complex128 psi (config 2 is complex, Fe2S2-OO-dcut-20.py:39) and a skewed table
+    # variants (the same step, --steps timed steps each): complex128 psi (config 2 is complex, Fe2S2-OO-dcut-20.py:39) and a skewed table
     variants = {}
-    vsteps, vwarm = max(3, min(args.steps, 5)), 3
+    vsteps, vwarm = args.steps, 3
     if not args.no_variants and world == 1:
         psi_c = make_psi(n_total, True)
         variants["complex128"] = (measure(keys_np, psi_c, vsteps, vwarm, want_e2e=False), keys_np, psi_c)
@@ -527,6 +533,33 @@ def run_ours(args):
             os._exit(3)
         sys.exit(3)
     leave(world)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, last: dict, rank: int, world: int) -> None:
+    """Write what the last timed step returned to its caller, as float64 .npy files in out_dir:
+      eloc.npy, psi0.npy     this rank's rows of the sorted table ([n] real, or [n, 2] = (re, im) for complex psi);
+      energy_statistics.npy  [mean.real, mean.imag, var, sd, se, n].
+    Above DUMP_BYTES in all, a fixed seeded sample of rows is written instead, with its row numbers in rows.npy.
+    With more than one rank, every rank writes its own files with a _rank<r> suffix."""
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    arrays = {k: np.ascontiguousarray(last[k]) for k in ("eloc", "psi0")}
+    arrays = {k: (a.view(np.float64).reshape(-1, 2) if np.iscomplexobj(a) else a).astype(np.float64) for k, a in arrays.items()}
+    n = arrays["eloc"].shape[0]
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    budget = DUMP_BYTES // world - 4096
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=budget // (row_bytes + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    st = last["stats"]
+    mean = complex(st["mean"])
+    arrays["energy_statistics"] = np.array([mean.real, mean.imag, st["var"], st["sd"], st["se"], st["n"]], dtype=np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}{sfx}.npy"), a)
 
 
 def leave(world: int) -> None:
@@ -650,7 +683,11 @@ def main():
     ap.add_argument("--table", default="uniform", help="sample set of the main measurement: uniform (the headline) or zipf0.8")
     ap.add_argument("--no-graph", action="store_true", help="launch the step kernel by kernel instead of replaying its CUDA graph")
     ap.add_argument("--no-peer", action="store_true", help="NCCL collectives only (no NVLink peer-memory pull kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the E_loc, psi0 and energy statistics of the last timed step "
+                                                          "as .npy files in DIR (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl != "ours":
         run_reference_arm(args)
     else:
