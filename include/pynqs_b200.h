@@ -151,6 +151,24 @@ int pynqs_eloc_sample_space(const uint8_t *bra, int64_t n, const double *h1e, co
                             int64_t N, const void *group_ws, void *scratch, int64_t scratch_bytes, void *eloc,
                             void *psi0, void *stream);
 
+/* Additive op: the sample-space Hamiltonian H[i, j] = <bra_i|H|key_j> (i < n, j < N) as a CSR matrix -- what the dense
+ * get_hij_torch(bra, key) (pynqs_hij, ket3d == 0) gives, without its n x N array.  Row i holds exactly the table rows that
+ * pynqs_eloc_sample_space sums over for bra_i: bra_i itself (if it is in the table) and its single and double excitations
+ * that are in the table; entries are structural (an element equal to 0.0 is stored), the columns of a row strictly
+ * ascending, the values bit-identical to pynqs_hij.  A table with duplicate keys gives the column the classic binary
+ * search lands on.  Same count / emit protocol as pynqs_reduce_count / _emit:
+ *   pynqs_hamiltonian_count: offsets int64[n + 1] = exclusive prefix of the row lengths, offsets[n] = nnz;
+ *   pynqs_hamiltonian_emit : col int64[nnz] and val double[nnz] of every row at those offsets (nnz = offsets[n], read by
+ *                            the caller).
+ * key / group_ws as for pynqs_eloc_sample_space.  scratch: pynqs_hamiltonian_scratch_bytes(n, nnz, ...) bytes -- size it
+ * for nnz = 0 before the count call and for the real nnz before the emit call. */
+int pynqs_hamiltonian_scratch_bytes(int64_t n, int64_t nnz, int sorb, int noA, int noB, int64_t *bytes);
+int pynqs_hamiltonian_count(const uint8_t *bra, int64_t n, int sorb, int noA, int noB, const uint8_t *key, int64_t N,
+                            const void *group_ws, void *scratch, int64_t scratch_bytes, int64_t *offsets, void *stream);
+int pynqs_hamiltonian_emit(const uint8_t *bra, int64_t n, const double *h1e, const double *h2e, int sorb, int nele, int noA,
+                           int noB, const uint8_t *key, int64_t N, const void *group_ws, void *scratch, int64_t scratch_bytes,
+                           const int64_t *offsets, int64_t nnz, int64_t *col, double *val, void *stream);
+
 /* ---- REDUCE method (vmc/energy/eloc.py:257-297, additive) -----------------------------------------
  * The reference materialises comb [n, M, 8L] and Hmat [n, M] and keeps torch.where(|Hmat| >= eps).  These
  * entry points return the kept rows only, in the same (ascending flat index s * M + m) order:
@@ -237,7 +255,8 @@ int pynqs_weighted_moments(const void *eloc, int eloc_complex, const void *weigh
  * block kernel, default 8), "eval_tiles" (evaluation kernel: 0 one warp per sample, 1 = default: 32 samples per warp for
  * large calls, 2: for every call), "block_parts" (block kernel: 0 = by the size of the call, 1 / 2 / 4: parts the groups
  * of a tile are split into), "lut_pipeline" (wavefunction_lut on one-word ONVs: 1 = default, four consecutive queries per
- * thread; 0: one query per thread).  name == NULL restores every default.  The scratch size of pynqs_eloc_scratch_bytes
+ * thread; 0: one query per thread), "sort_chunk" (pynqs_hamiltonian_emit: 0 = default, rows sorted in as few calls as
+ * 31-bit offsets allow; else the calls take the rows starting in windows of this many entries).  name == NULL restores every default.  The scratch size of pynqs_eloc_scratch_bytes
  * depends on the knobs: set them before sizing the scratch. */
 int pynqs_set_tuning(const char *name, int64_t value);
 

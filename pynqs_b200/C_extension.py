@@ -618,6 +618,57 @@ def eloc_sample_space(
     return eloc, psi0
 
 
+def sample_space_hamiltonian(
+    bra: Tensor, h1e: Tensor, h2e: Tensor, sorb: int, nele: int, noA: int, noB: int,
+    bra_key: Tensor, group_index: GroupIndex | None = None,
+) -> Tuple[Tensor, Tensor, Tensor]:
+    """Additive op: H[i, j] = <bra_i|H|bra_key_j> as CSR arrays (crow int64 [n + 1], col int64 [nnz], val float64 [nnz]) --
+    the rows of get_hij_torch(bra, bra_key) restricted to the entries eloc_sample_space sums over: bra_i itself (when it is in
+    the table) and its single and double excitations that are in the table.  Entries are structural (exact zeros are kept),
+    columns ascend within a row, values are bit-identical to get_hij_torch.  One host synchronisation (nnz)."""
+    dev = _need_cuda(bra, h1e, h2e, bra_key)
+    for t, nm in ((bra, "bra"), (h1e, "h1e"), (h2e, "h2e"), (bra_key, "bra_key")):
+        _contig(t, nm)
+    if bra.dim() != 2 or bra_key.dim() != 2:
+        raise ValueError("bra and bra_key must be 2-D [rows, 8L]")
+    L = _check_width(bra, sorb, "bra")
+    if _onv_words(bra_key, "bra_key") != L:
+        raise ValueError("bra and bra_key widths differ")
+    if h1e.dtype != torch.float64 or h2e.dtype != torch.float64:
+        raise ValueError("sample_space_hamiltonian needs float64 integrals")
+    _check_integrals(h1e, h2e, sorb)
+    get_Num_SinglesDoubles(sorb, noA, noB)  # geometry / overflow checks
+    n, N = bra.size(0), bra_key.size(0)
+    crow = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+    if n == 0 or N == 0:
+        return crow, torch.empty(0, dtype=torch.int64, device=dev), torch.empty(0, dtype=torch.float64, device=dev)
+    if group_index is None:
+        group_index = _cached_group(bra_key)
+    if group_index.N != N or group_index.L != L or group_index.key_ptr != bra_key.data_ptr():
+        raise ValueError("group_index was built for another key table")
+    lib = _lib.load()
+
+    def scratch_for(nnz: int) -> Tensor:
+        nbytes = _lib.ctypes.c_int64()
+        _lib.check(lib.pynqs_hamiltonian_scratch_bytes(i64(n), i64(nnz), int(sorb), int(noA), int(noB), _lib.ctypes.byref(nbytes)))
+        return torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+
+    table = (vp(bra_key.data_ptr()), i64(N), vp(group_index.workspace.data_ptr()))
+    with torch.cuda.device(dev):
+        scratch = scratch_for(0)
+        _lib.check(lib.pynqs_hamiltonian_count(vp(bra.data_ptr()), i64(n), int(sorb), int(noA), int(noB), *table, vp(scratch.data_ptr()),
+                                               i64(scratch.numel()), vp(crow.data_ptr()), _stream(dev)))
+        nnz = int(crow[n].item())
+        del scratch
+        scratch = scratch_for(nnz)
+        col = torch.empty(nnz, dtype=torch.int64, device=dev)
+        val = torch.empty(nnz, dtype=torch.float64, device=dev)
+        _lib.check(lib.pynqs_hamiltonian_emit(vp(bra.data_ptr()), i64(n), vp(h1e.data_ptr()), vp(h2e.data_ptr()), int(sorb), int(nele),
+                                              int(noA), int(noB), *table, vp(scratch.data_ptr()), i64(scratch.numel()), vp(crow.data_ptr()),
+                                              i64(nnz), vp(col.data_ptr()), vp(val.data_ptr()), _stream(dev)))
+    return crow, col, val
+
+
 def lookup_compact(idx_array: Tensor, mask: Tensor, wf_value: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
     """(positions with mask set, positions without, wf_value[idx_array[mask]]) -- the index glue of
     WavefunctionLUT.lookup (utils/public_function.py:825-838: arange, two boolean-mask selections, masked_select, gather)

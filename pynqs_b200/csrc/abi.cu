@@ -53,6 +53,9 @@ long long group_workspace_bytes(long long, int);
 int launch_group_build(const u64 *, long long, int, void *, long long, cudaStream_t);
 int launch_eloc(const u64 *, long long, const double *, const double *, const u64 *, const double *, int, long long,
                 const void *, void *, long long, double *, double *, const ExcGeom &, cudaStream_t);
+long long hamiltonian_scratch_bytes(long long, long long, const ExcGeom &);
+int launch_hamiltonian(const u64 *, long long, const double *, const double *, const u64 *, long long, const void *, void *, long long,
+                       long long *, long long, long long *, double *, const ExcGeom &, int, cudaStream_t);
 long long sort_workspace_bytes(long long);
 int launch_sort_table(const u64 *, const void *, long long, int, int, int, u64 *, void *, long long *, void *, long long, cudaStream_t);
 long long moments_scratch_bytes();
@@ -360,7 +363,8 @@ int pynqs_set_tuning(const char *name, int64_t value) {
                {"full_keys", &t.full_keys, 0, 1},                {"block_min_samples", &t.block_min_samples, 1, 1LL << 30},
                {"block_min_group", &t.block_min_group, 4, 32},   {"block_enable", &t.block_enable, 0, 1},
                {"eval_tiles", &t.eval_tiles, 0, 2},
-               {"lut_pipeline", &t.lut_pipeline, 0, 1},          {"block_parts", &t.block_parts, 0, 4}};
+               {"lut_pipeline", &t.lut_pipeline, 0, 1},          {"block_parts", &t.block_parts, 0, 4},
+               {"sort_chunk", &t.sort_chunk, 0, 1LL << 30}};
   if (name == nullptr) {
     t = ElocTuning();  // back to the production values
     return 0;
@@ -399,6 +403,39 @@ int pynqs_eloc_sample_space(const uint8_t *bra, int64_t n, const double *h1e, co
   return launch_eloc(reinterpret_cast<const u64 *>(bra), n, h1e, h2e, reinterpret_cast<const u64 *>(key),
                      (const double *)psi, psi_complex, N, group_ws, scratch, scratch_bytes, (double *)eloc, (double *)psi0, g,
                      (cudaStream_t)stream);
+}
+
+int pynqs_hamiltonian_scratch_bytes(int64_t n, int64_t nnz, int sorb, int noA, int noB, int64_t *bytes) {
+  if (int rc = check_geometry(sorb, 0, noA, noB)) return rc;
+  long long nsd;
+  if (int rc = num_sd_checked(sorb, noA, noB, &nsd)) return rc;
+  if (n < 0 || nnz < 0) {
+    set_error("hamiltonian_scratch_bytes: bad n = %lld or nnz = %lld", (long long)n, (long long)nnz);
+    return PYNQS_EVALUE;
+  }
+  *bytes = hamiltonian_scratch_bytes(n, nnz, make_geom(sorb, noA + noB, noA, noB));
+  return 0;
+}
+
+int pynqs_hamiltonian_count(const uint8_t *bra, int64_t n, int sorb, int noA, int noB, const uint8_t *key, int64_t N, const void *group_ws,
+                            void *scratch, int64_t scratch_bytes, int64_t *offsets, void *stream) {
+  if (int rc = check_geometry(sorb, noA + noB, noA, noB)) return rc;
+  long long nsd;
+  if (int rc = num_sd_checked(sorb, noA, noB, &nsd)) return rc;
+  return launch_hamiltonian(reinterpret_cast<const u64 *>(bra), n, nullptr, nullptr, reinterpret_cast<const u64 *>(key), N, group_ws, scratch,
+                            scratch_bytes, reinterpret_cast<long long *>(offsets), 0, nullptr, nullptr, make_geom(sorb, noA + noB, noA, noB),
+                            0, (cudaStream_t)stream);
+}
+
+int pynqs_hamiltonian_emit(const uint8_t *bra, int64_t n, const double *h1e, const double *h2e, int sorb, int nele, int noA, int noB,
+                           const uint8_t *key, int64_t N, const void *group_ws, void *scratch, int64_t scratch_bytes, const int64_t *offsets,
+                           int64_t nnz, int64_t *col, double *val, void *stream) {
+  if (int rc = check_geometry(sorb, nele, noA, noB)) return rc;
+  long long nsd;
+  if (int rc = num_sd_checked(sorb, noA, noB, &nsd)) return rc;
+  return launch_hamiltonian(reinterpret_cast<const u64 *>(bra), n, h1e, h2e, reinterpret_cast<const u64 *>(key), N, group_ws, scratch,
+                            scratch_bytes, const_cast<long long *>(reinterpret_cast<const long long *>(offsets)), nnz,
+                            reinterpret_cast<long long *>(col), val, make_geom(sorb, nele, noA, noB), 1, (cudaStream_t)stream);
 }
 
 int64_t pynqs_reduce_scratch_bytes(int64_t n) { return reduce_scratch_bytes(n); }

@@ -997,22 +997,13 @@ int block_run_stride();
 int launch_eloc_block(const u64 *bra, long long n, const GroupView &gv, char *block_ws, ElocCounters *ctr, HitRun *runs, u32 *run_cnt,
                       int run_stride, u32 *hits, u32 *self_pos, u32 hit_cap, const ExcGeom &g, const u32 **slots_out, cudaStream_t st);
 
-struct ElocScratch {
-  long long hii, self_pos, run_cnt, heavy, runs, counters, block_ws, hits, total;
-  long long hit_cap, batch;
-  int splits;      // same for every batch of the call (sized for the first, largest one)
-  int warps;       // warps per scan CTA
-  int run_stride;  // HitRun records per sample
-  bool block;      // samples grouped by beta string first (eloc_block.cu); the per-sample kernel takes the rest
-};
-
 // the block route needs one-word ONVs (decided again at launch: it also needs N < 2^30 and the folded route)
-static bool block_route_wanted(long long n, const ExcGeom &g) {
+bool block_route_wanted(long long n, const ExcGeom &g) {
   const ElocTuning &t = eloc_tuning();
   return t.block_enable && !t.full_keys && g.L == 1 && n >= t.block_min_samples && g.noB * g.nvB + 2 <= 258;
 }
 
-static ElocScratch eloc_scratch_layout(long long n, const ExcGeom &g, bool block) {
+ElocScratch eloc_scratch_layout(long long n, const ExcGeom &g, bool block) {
   ElocScratch l;
   l.block = block;
   l.warps = scan_threads(g.noB * g.nvB + 2) / 32;
@@ -1060,17 +1051,13 @@ long long eloc_scratch_bytes(long long n, const ExcGeom &g) {
   return t;
 }
 
-int launch_diag_f64(const u64 *bra, const double *h1e, const double *h2e, double *out, long long n, long long stride, int L,
-                    int sorb, int nele, cudaStream_t st);
-
-template <int L, bool CPLX, bool HALF>
-static int launch_eloc_LC(const u64 *bra, long long n, const double *h1e, const double *h2e, const u64 *key, const double *psi,
-                          long long N, const GroupView &gv, char *scratch, const ElocScratch &lay, double *eloc, double *psi0,
-                          const ExcGeom &g, cudaStream_t st, SideLane *diag_lane) {
-  double *hii = reinterpret_cast<double *>(scratch + lay.hii);
+// The scan phase of one batch of samples bra[0, nb): the grouping pass and the block kernel (block route), then the
+// per-sample scan kernel.  Leaves the batch's hit lists in the scratch (runs, run_cnt, hits, self_pos).
+template <int L, bool HALF>
+static int scan_batch(const u64 *bra, long long nb, const GroupView &gv, char *scratch, const ElocScratch &lay, const ExcGeom &g,
+                      cudaStream_t st) {
   u32 *self_pos = reinterpret_cast<u32 *>(scratch + lay.self_pos);
   u32 *run_cnt = reinterpret_cast<u32 *>(scratch + lay.run_cnt);
-  u32 *heavy = reinterpret_cast<u32 *>(scratch + lay.heavy);
   HitRun *runs = reinterpret_cast<HitRun *>(scratch + lay.runs);
   ElocCounters *ctr = reinterpret_cast<ElocCounters *>(scratch + lay.counters);
   u32 *hits = reinterpret_cast<u32 *>(scratch + lay.hits);
@@ -1085,27 +1072,55 @@ static int launch_eloc_LC(const u64 *bra, long long n, const double *h1e, const 
   auto scan = lay.warps == 2 ? eloc_scan_kernel<L, HALF, 64> : (lay.warps == 4 ? eloc_scan_kernel<L, HALF, 128> : eloc_scan_kernel<L, HALF, 256>);
   if (smem > 48 * 1024 && cudaFuncSetAttribute(scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return check_launch("eloc_scan_kernel smem opt-in");
+  const int splits = lay.splits;
+  if (cudaMemsetAsync(ctr, 0, sizeof(ElocCounters), st) != cudaSuccess) return check_launch("eloc counters memset");
+  if (cudaMemsetAsync(self_pos, 0xff, 4 * (size_t)nb, st) != cudaSuccess) return check_launch("eloc self memset");
+  const u32 *ids = nullptr;
+  unsigned grid = (unsigned)(nb * splits);
+  if (HALF && lay.block) {
+    // samples that share a beta string with enough others: tiles of the block kernel; the rest: per-sample kernel,
+    // which finds its work list (and its length) in device memory -- a fixed grid of persistent CTAs
+    if (int rc = launch_eloc_block(bra, nb, gv, scratch + lay.block_ws, ctr, runs, run_cnt, lay.run_stride, hits, self_pos,
+                                   (u32)lay.hit_cap, g, &ids, st))
+      return rc;
+    const long long cap = 148LL * 12;
+    grid = (unsigned)(nb < cap ? nb : cap);
+  }
+  scan<<<grid, lay.warps * 32, smem, st>>>(bra, nb, gv, runs, run_cnt, lay.run_stride, hits, self_pos, ctr, (u32)lay.hit_cap, splits, ids,
+                                           g, sm);
+  count_launch();
+  return check_launch("eloc_scan_kernel");
+}
+
+int launch_scan_batch(const u64 *bra, long long nb, const GroupView &gv, char *scratch, const ElocScratch &lay, const ExcGeom &g, bool half,
+                      cudaStream_t st) {
+  if (half) return scan_batch<1, true>(bra, nb, gv, scratch, lay, g, st);
+  switch (g.L) {
+    case 1: return scan_batch<1, false>(bra, nb, gv, scratch, lay, g, st);
+    case 2: return scan_batch<2, false>(bra, nb, gv, scratch, lay, g, st);
+    case 3: return scan_batch<3, false>(bra, nb, gv, scratch, lay, g, st);
+  }
+  set_error("unsupported ONV length L=%d", g.L);
+  return 1;
+}
+
+bool eloc_half_route(long long N, const ExcGeom &g) { return g.L == 1 && N < (1LL << 30) && !eloc_tuning().full_keys; }
+
+template <int L, bool CPLX, bool HALF>
+static int launch_eloc_LC(const u64 *bra, long long n, const double *h1e, const double *h2e, const u64 *key, const double *psi,
+                          long long N, const GroupView &gv, char *scratch, const ElocScratch &lay, double *eloc, double *psi0,
+                          const ExcGeom &g, cudaStream_t st, SideLane *diag_lane) {
+  double *hii = reinterpret_cast<double *>(scratch + lay.hii);
+  u32 *self_pos = reinterpret_cast<u32 *>(scratch + lay.self_pos);
+  u32 *run_cnt = reinterpret_cast<u32 *>(scratch + lay.run_cnt);
+  u32 *heavy = reinterpret_cast<u32 *>(scratch + lay.heavy);
+  HitRun *runs = reinterpret_cast<HitRun *>(scratch + lay.runs);
+  ElocCounters *ctr = reinterpret_cast<ElocCounters *>(scratch + lay.counters);
+  u32 *hits = reinterpret_cast<u32 *>(scratch + lay.hits);
   const int w = CPLX ? 2 : 1;
   for (long long b0 = 0; b0 < n; b0 += lay.batch) {
     const long long nb = n - b0 < lay.batch ? n - b0 : lay.batch;
-    const int splits = lay.splits;
-    if (cudaMemsetAsync(ctr, 0, sizeof(ElocCounters), st) != cudaSuccess) return check_launch("eloc counters memset");
-    if (cudaMemsetAsync(self_pos, 0xff, 4 * (size_t)nb, st) != cudaSuccess) return check_launch("eloc self memset");
-    const u32 *ids = nullptr;
-    unsigned grid = (unsigned)(nb * splits);
-    if (HALF && lay.block) {
-      // samples that share a beta string with enough others: tiles of the block kernel; the rest: per-sample kernel,
-      // which finds its work list (and its length) in device memory -- a fixed grid of persistent CTAs
-      if (int rc = launch_eloc_block(bra + b0 * L, nb, gv, scratch + lay.block_ws, ctr, runs, run_cnt, lay.run_stride, hits, self_pos,
-                                     (u32)lay.hit_cap, g, &ids, st))
-        return rc;
-      const long long cap = 148LL * 12;
-      grid = (unsigned)(nb < cap ? nb : cap);
-    }
-    scan<<<grid, lay.warps * 32, smem, st>>>(bra + b0 * L, nb, gv, runs, run_cnt, lay.run_stride, hits, self_pos, ctr, (u32)lay.hit_cap,
-                                             splits, ids, g, sm);
-    count_launch();
-    if (int rc = check_launch("eloc_scan_kernel")) return rc;
+    if (int rc = scan_batch<L, HALF>(bra + b0 * L, nb, gv, scratch, lay, g, st)) return rc;
     if (diag_lane != nullptr) {  // the diagonal elements (side stream) must be there now
       if (!side_join(diag_lane, st)) return check_launch("eloc: join of the diagonal kernel");
       diag_lane = nullptr;
@@ -1144,7 +1159,7 @@ int launch_eloc(const u64 *bra, long long n, const double *h1e, const double *h2
   if (n == 0) return 0;
   // folded 32-bit strings: one-word ONVs, two flag bits in the hit word.  The tuning knob full_keys forces the
   // full-key route (the one multi-word ONVs take) -- used by the parity tests to cover both.
-  const bool half = g.L == 1 && N < (1LL << 30) && !eloc_tuning().full_keys;
+  const bool half = eloc_half_route(N, g);
   const ElocScratch lay = eloc_scratch_layout(n, g, half && block_route_wanted(n, g));
   if (scratch_bytes < lay.total) {
     set_error("eloc scratch too small: %lld < %lld bytes", scratch_bytes, lay.total);

@@ -49,6 +49,18 @@ def local_energy_sample_space(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: Wavef
     return eloc.to(dtype), torch.zeros_like(eloc).to(dtype), psi0.to(dtype)
 
 
+def sample_space_hamiltonian(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: WavefunctionLUT, sorb: int, nele: int,
+                             noa: int, nob: int) -> Tensor:
+    """H[i, j] = <x_i|H|WF_LUT.bra_key[j]> as a float64 torch.sparse_csr_tensor of shape [n, N]: the connections that
+    local_energy_sample_space sums over, so (H @ psi)[i] = eloc[i] * psi_x[i] with psi = WF_LUT.wf_value.  With x = the
+    table itself it is the square sample-space Hamiltonian (variational energy psi^T H psi / psi^T psi, selected-CI
+    diagonalisation, many products H psi without rescanning)."""
+    N = WF_LUT.bra_key.size(0)
+    crow, col, val = ops.sample_space_hamiltonian(x, h1e, h2e, sorb, nele, noa, nob, WF_LUT.bra_key,
+                                                  WF_LUT.group_index if N > 0 else None)
+    return torch.sparse_csr_tensor(crow, col, val, size=(x.size(0), N))
+
+
 def local_energy_three_call(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: WavefunctionLUT, sorb: int, nele: int,
                             noa: int, nob: int, dtype=torch.double, batch: int = 4096) -> Tuple[Tensor, Tensor, Tensor]:
     """The reference's op sequence (eloc.py:369-397) in chunks of `batch` samples."""
