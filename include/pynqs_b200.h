@@ -169,6 +169,16 @@ int pynqs_hamiltonian_emit(const uint8_t *bra, int64_t n, const double *h1e, con
                            int noB, const uint8_t *key, int64_t N, const void *group_ws, void *scratch, int64_t scratch_bytes,
                            const int64_t *offsets, int64_t nnz, int64_t *col, double *val, void *stream);
 
+/* Additive op: Y = H X for a CSR matrix H laid out as pynqs_hamiltonian_emit writes it (crow int64[n + 1], col int64[nnz]
+ * with columns < N, val double[nnz]; nnz = crow[n] is read on the device only) and row-major blocks X double[N, k] (row
+ * stride ldx) and Y double[n, k] (row stride ldy), 1 <= k <= 8: Y[i, c] = sum over the entries p of row i of
+ * val[p] * X[col[p], c].  Wider blocks go through in column slices (X + c0, Y + c0, same ld).  Deterministic: each Y[i, c]
+ * is summed in an order fixed by the length of row i, so two calls give identical bits.  Empty rows give 0.  PYNQS_EVALUE,
+ * before anything touches the device, for n < 0, N < 0, k outside [1, 8], ldx < k, ldy < k, or a NULL crow / Y (n > 0) or
+ * col / val / X (n > 0 and N > 0).  n == 0 launches nothing. */
+int pynqs_csr_spmm(const int64_t *crow, const int64_t *col, const double *val, int64_t n, int64_t N, const double *X, int64_t ldx, int k,
+                   double *Y, int64_t ldy, void *stream);
+
 /* ---- REDUCE method (vmc/energy/eloc.py:257-297, additive) -----------------------------------------
  * The reference materialises comb [n, M, 8L] and Hmat [n, M] and keeps torch.where(|Hmat| >= eps).  These
  * entry points return the kept rows only, in the same (ascending flat index s * M + m) order:

@@ -669,6 +669,48 @@ def sample_space_hamiltonian(
     return crow, col, val
 
 
+def csr_matmul(crow: Tensor, col: Tensor, val: Tensor, X: Tensor, N: int) -> Tensor:
+    """Y = H X for the CSR matrix H [n, N] of sample_space_hamiltonian (crow int64 [n + 1], col int64 [nnz] < N, val float64
+    [nnz]).  X: float64 or complex128, [N] or [N, k] of any k (rows may be strided, columns must be adjacent or X is
+    copied); Y has X's dtype and shape with n rows.  H is real, so a complex X is multiplied as its torch.view_as_real
+    view, real and imaginary parts in one pass.  The kernel takes 8 columns per call; wider blocks go through in column
+    slices of X and Y.  Deterministic (identical bits on every call); no host synchronisation."""
+    dev = _need_cuda(crow, col, val, X)
+    if crow.dtype != torch.int64 or col.dtype != torch.int64 or val.dtype != torch.float64:
+        raise ValueError("crow and col must be int64, val float64")
+    if crow.dim() != 1 or crow.numel() < 1 or col.dim() != 1 or val.shape != col.shape:
+        raise ValueError("crow must be 1-D [n + 1], col and val 1-D of the same length")
+    for t, nm in ((crow, "crow"), (col, "col"), (val, "val")):
+        _contig(t, nm)
+    if X.dtype not in (torch.float64, torch.complex128):
+        raise ValueError(f"X must be float64 or complex128, got {X.dtype}")
+    N = int(N)
+    if X.dim() not in (1, 2) or X.size(0) != N:
+        raise ValueError(f"X must be [N] or [N, k] with N = {N}, got {tuple(X.shape)}")
+    n = crow.numel() - 1
+    Xr = X.unsqueeze(1) if X.dim() == 1 else X
+    if (Xr.size(1) > 1 and Xr.stride(1) != 1) or (N > 1 and Xr.stride(0) < Xr.size(1)):
+        Xr = Xr.contiguous()  # the kernel reads rows of adjacent columns, rows apart by ldx >= k
+    if X.is_complex():
+        Xr = torch.view_as_real(Xr.resolve_conj())
+        Xr = Xr.as_strided((N, 2 * Xr.size(1)), (Xr.stride(0), 1))  # [N, k, 2] with adjacent columns -> real [N, 2k]
+    kk = Xr.size(1)
+    ldx = Xr.stride(0) if N > 1 else kk  # a single row's stride is not meaningful
+    work = n > 0 and N > 0 and col.numel() > 0 and kk > 0
+    Y = (torch.empty if work else torch.zeros)((n, kk), dtype=torch.float64, device=dev)
+    if work:
+        lib = _lib.load()
+        with torch.cuda.device(dev):
+            for c0 in range(0, kk, 8):
+                k = min(8, kk - c0)
+                _lib.check(lib.pynqs_csr_spmm(vp(crow.data_ptr()), vp(col.data_ptr()), vp(val.data_ptr()), i64(n), i64(N),
+                                              vp(Xr.data_ptr() + 8 * c0), i64(ldx), int(k), vp(Y.data_ptr() + 8 * c0), i64(kk),
+                                              _stream(dev)))
+    if X.is_complex():
+        Y = torch.view_as_complex(Y.view(n, kk // 2, 2))
+    return Y.view(n) if X.dim() == 1 else Y
+
+
 def lookup_compact(idx_array: Tensor, mask: Tensor, wf_value: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
     """(positions with mask set, positions without, wf_value[idx_array[mask]]) -- the index glue of
     WavefunctionLUT.lookup (utils/public_function.py:825-838: arange, two boolean-mask selections, masked_select, gather)

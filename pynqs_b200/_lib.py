@@ -15,7 +15,7 @@ SYMBOLS = [
     "pynqs_comb_hij_fused", "pynqs_hij",
     "pynqs_lut", "pynqs_hash_bytes", "pynqs_hash_build", "pynqs_lut_hashed",
     "pynqs_group_bytes", "pynqs_group_build", "pynqs_group_layout", "pynqs_eloc_scratch_bytes", "pynqs_eloc_sample_space",
-    "pynqs_hamiltonian_scratch_bytes", "pynqs_hamiltonian_count", "pynqs_hamiltonian_emit",
+    "pynqs_hamiltonian_scratch_bytes", "pynqs_hamiltonian_count", "pynqs_hamiltonian_emit", "pynqs_csr_spmm",
     "pynqs_reduce_scratch_bytes", "pynqs_reduce_count", "pynqs_reduce_emit", "pynqs_reduce_eloc",
     "pynqs_reduce_sample_scratch_bytes", "pynqs_reduce_sample_count", "pynqs_reduce_sample_emit",
     "pynqs_compact_scratch_bytes", "pynqs_lookup_count", "pynqs_lookup_emit", "pynqs_unique_count", "pynqs_unique_emit",

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libpynqs_b200.so")
-SOURCES = ["abi.cu", "enumerate.cu", "hij.cu", "lut.cu", "eloc_scan.cu", "eloc_block.cu", "hamiltonian.cu", "gindex.cu", "convert.cu", "reduce_sample.cu", "compact.cu", "peer.cu", "prepare.cu", "table.cu"]
+SOURCES = ["abi.cu", "enumerate.cu", "hij.cu", "lut.cu", "eloc_scan.cu", "eloc_block.cu", "hamiltonian.cu", "spmm.cu", "gindex.cu", "convert.cu", "reduce_sample.cu", "compact.cu", "peer.cu", "prepare.cu", "table.cu"]
 HEADERS = ["common.cuh", "lut.cuh", "tables.cuh", "prepare.cuh", "gindex.cuh", "eloc.cuh", "rederive.cuh", os.path.join("..", "..", "include", "pynqs_b200.h")]
 
 NVCC_FLAGS = [

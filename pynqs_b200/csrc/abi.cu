@@ -81,6 +81,8 @@ int launch_peer_gather_rows(const void *const *, long long, const u32 *, long lo
 int launch_merge_counts(const long long *, const long long *, long long, long long, long long *, cudaStream_t);
 int launch_onv_to_tensor(const u64 *, void *, int, long long, int, cudaStream_t);
 int launch_tensor_to_onv(const unsigned char *, unsigned char *, long long, int, cudaStream_t);
+int launch_csr_spmm(const long long *, const long long *, const double *, long long, const double *, long long, int, double *, long long,
+                    cudaStream_t);
 
 static int check_geometry(int sorb, int nele, int noA, int noB) {
   if (sorb <= 0 || sorb > PYNQS_MAX_SORB) {
@@ -436,6 +438,22 @@ int pynqs_hamiltonian_emit(const uint8_t *bra, int64_t n, const double *h1e, con
   return launch_hamiltonian(reinterpret_cast<const u64 *>(bra), n, h1e, h2e, reinterpret_cast<const u64 *>(key), N, group_ws, scratch,
                             scratch_bytes, const_cast<long long *>(reinterpret_cast<const long long *>(offsets)), nnz,
                             reinterpret_cast<long long *>(col), val, make_geom(sorb, nele, noA, noB), 1, (cudaStream_t)stream);
+}
+
+int pynqs_csr_spmm(const int64_t *crow, const int64_t *col, const double *val, int64_t n, int64_t N, const double *X, int64_t ldx, int k,
+                   double *Y, int64_t ldy, void *stream) {
+  if (n < 0 || N < 0 || k < 1 || k > 8 || ldx < k || ldy < k) {
+    set_error("csr_spmm: bad n = %lld, N = %lld, k = %d, ldx = %lld or ldy = %lld (k in [1, 8], ld >= k)", (long long)n, (long long)N, k,
+              (long long)ldx, (long long)ldy);
+    return PYNQS_EVALUE;
+  }
+  if (n > 0 && (crow == nullptr || Y == nullptr || (N > 0 && (col == nullptr || val == nullptr || X == nullptr)))) {
+    set_error("csr_spmm: null pointer (crow / Y for n > 0, col / val / X as well for N > 0)");
+    return PYNQS_EVALUE;
+  }
+  if (n == 0) return 0;
+  return launch_csr_spmm(reinterpret_cast<const long long *>(crow), reinterpret_cast<const long long *>(col), val, n, X, ldx, k, Y, ldy,
+                         (cudaStream_t)stream);
 }
 
 int64_t pynqs_reduce_scratch_bytes(int64_t n) { return reduce_scratch_bytes(n); }

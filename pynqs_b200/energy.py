@@ -17,6 +17,7 @@ import torch
 from torch import Tensor
 
 from . import C_extension as ops
+from .davidson import davidson
 from .lut import WavefunctionLUT
 
 
@@ -59,6 +60,29 @@ def sample_space_hamiltonian(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: Wavefu
     crow, col, val = ops.sample_space_hamiltonian(x, h1e, h2e, sorb, nele, noa, nob, WF_LUT.bra_key,
                                                   WF_LUT.group_index if N > 0 else None)
     return torch.sparse_csr_tensor(crow, col, val, size=(x.size(0), N))
+
+
+def sample_space_ground_state(WF_LUT: WavefunctionLUT, h1e: Tensor, h2e: Tensor, sorb: int, nele: int, noa: int, nob: int,
+                              nroots: int = 1, *, H: "Tensor | None" = None, guess: "Tensor | None" = None, tol: float = 1e-8,
+                              max_iter: int = 200) -> Tuple[Tensor, Tensor, dict]:
+    """The lowest `nroots` eigenpairs of the square sample-space Hamiltonian over the determinants of WF_LUT.bra_key: the
+    variational energies within the sample set and their CI coefficients.  Block Davidson (pynqs_b200.davidson) with
+    H X = C_extension.csr_matmul on the device CSR matrix and the diagonal <x|H|x> as preconditioner.
+
+    H: sample_space_hamiltonian(WF_LUT.bra_key, ...) (built when not given; pass it to reuse it).  guess: [N] or [N, b] start
+    vectors, e.g. the real part of a VMC psi (default: unit vectors on the nroots lowest diagonal entries, ties broken by
+    table row).  Returns (energies [nroots] ascending, electronic like eloc; coeffs [N, nroots] orthonormal, rows in the
+    order of WF_LUT.bra_key; info of davidson: iterations, products, residual_norms, converged)."""
+    keys = WF_LUT.bra_key
+    N = keys.size(0)
+    if H is None:
+        H = sample_space_hamiltonian(keys, h1e, h2e, WF_LUT, sorb, nele, noa, nob)
+    if H.layout != torch.sparse_csr or tuple(H.shape) != (N, N):
+        raise ValueError(f"H must be a sparse CSR tensor of shape ({N}, {N})")
+    crow, col, val = H.crow_indices(), H.col_indices(), H.values()
+    # <x|H|x> from the 3-D form: one ket per bra, bit-identical to the CSR diagonal, nothing of size nnz
+    diag = ops.get_hij_torch(keys, keys.view(N, 1, keys.size(1)), h1e, h2e, sorb, nele).view(N)
+    return davidson(lambda V: ops.csr_matmul(crow, col, val, V, N), diag, nroots, guess=guess, tol=tol, max_iter=max_iter)
 
 
 def local_energy_three_call(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: WavefunctionLUT, sorb: int, nele: int,
