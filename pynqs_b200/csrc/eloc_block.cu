@@ -7,15 +7,15 @@
 // of the samples inside a group is irrelevant), and one warp then takes a TILE of up to 32 samples with the same
 // beta string -- one sample per lane -- and walks the shared groups once for all of them:
 //
-//   * the folded alpha strings of the groups' keys are copied into shared memory with cp.async (coalesced, all
-//     copies of a fill in flight at once) and read back as broadcast LDS.128;
-//   * per key and per 32 samples the test is three instructions (XOR, POPC, compare-and-OR into a predicate);
-//     a lane only records WHICH block of 8 keys held a hit, the block is re-examined when the queue is flushed;
+//   * the groups are walked in chunks of 32 keys; the bit planes of a chunk (the 32 keys' folded alpha strings
+//     bit-transposed, GroupView::planes) are copied into shared memory with cp.async (coalesced, all copies of a fill in
+//     flight at once);
+//   * a lane reads the planes of its K = min(noA, nvA) orbitals and counts, for the 32 keys at once, how many of them
+//     are on the wrong side (~3 instructions per orbital): the result is the exact mask of its hits in the chunk;
 //   * bucket bounds, hashing, duplicate-bucket detection and the copy are paid once per tile, not per sample.
 //
-// Compared with the per-sample kernel (16 instructions per 32 key tests plus ~2 000 per sample of set-up) this is
-// ~4 instructions per 32 tests and ~100 per sample of set-up.  Groups with fewer than `block_min_group` samples stay
-// with the per-sample kernel (a lane-per-sample walk with one lane is slower than a lane-per-key walk).
+// Groups with fewer than `block_min_group` samples stay with the per-sample kernel (a lane-per-sample walk with one lane
+// is slower than a lane-per-key walk).
 //
 // The sample's own-alpha group (beta singles, beta-beta doubles) depends on the sample, not on the tile: it is walked
 // per sample with one key per lane, as in the per-sample kernel.
@@ -27,29 +27,21 @@
 
 namespace pynqs {
 
-constexpr int kBlkWarps = 4;     // warps per CTA; every warp works on its own tile
-#ifndef PYNQS_STAGE
-#define PYNQS_STAGE 512
-#endif
-#ifndef PYNQS_QCAP
-#define PYNQS_QCAP 32
-#endif
-constexpr int kStage = PYNQS_STAGE;  // folded strings staged per warp and fill
-constexpr int kQCap = PYNQS_QCAP;    // queue entries per lane (16-bit: index of a block of 8 staged keys)
-constexpr int kMaxGroups = 260;  // beta singles of a one-word ONV (<= 16 * 16) + the own group
-constexpr int kFirstBlock = 64;  // hit-buffer block sizes of a sample: 64, 128, ... (one HitRun each)
+constexpr int kBlkWarps = 4;       // warps per CTA; every warp works on its own tile
+constexpr int kStageChunks = 32;   // chunks of 32 keys whose bit planes are staged per warp and fill (4 KB)
+constexpr int kMaxGroups = 260;    // beta singles of a one-word ONV (<= 16 * 16) + the own group
+constexpr int kMaxOrbs = 16;       // orbitals a lane tests: min(noA, nvA) <= 32 / 2
+constexpr int kFirstBlock = 64;    // hit-buffer block sizes of a sample: 64, 128, ... (one HitRun each)
 
 struct BlockWarpSmem {
-  u32 stage[kStage];
-  unsigned short queue[kQCap * 32];  // [entry][lane]
-  uint2 rng[kMaxGroups];             // bucket [first, end) of every group; group sB = the tile's own beta string
-  u32 goff[kMaxGroups];              // first block (of 8 keys) of every group among the blocks of its walk
-  u32 blkpos[kStage / 8];            // position in the grouped copy of the first key of every staged block of 8
-  unsigned char blkcnt[kStage / 8];  // keys in the block (the rest is padding)
+  u32 stage[kStageChunks * 32];  // [chunk][folded orbital]: bit planes of the staged chunks
+  uint2 chunk[kStageChunks];     // of every staged chunk: its number (position / 32) and the mask of its keys in the group
+  uint2 rng[kMaxGroups];         // bucket [first, end) of every group; group sB = the tile's own beta string
+  u32 goff[kMaxGroups];          // first chunk of every group among the chunks of its walk
   unsigned char bpos[32];
 };
-constexpr int kDupSet = 512;  // open-addressing set of the bucket starts of a walk (lives in the idle queue)
-static_assert(kDupSet * 4 <= kQCap * 32 * 2 && kDupSet <= kStage && kDupSet >= 2 * 256, "duplicate-bucket set: twice the largest number of groups");
+constexpr int kDupSet = 512;  // open-addressing set of the bucket starts of a walk (lives in the idle stage, next to minq)
+static_assert(2 * kDupSet <= kStageChunks * 32 && kDupSet >= 2 * 256, "duplicate-bucket set: twice the largest number of groups");
 
 __host__ __device__ inline u32 sample_log2_buckets(long long n) {
   u32 lg = 10;
@@ -106,9 +98,8 @@ sample_scatter_kernel(const u64 *__restrict__ bra, long long n, u32 shift, u32 *
 // ---- the block kernel -------------------------------------------------------------------------------------------------
 struct BlockGeom {
   int sorb, noA, noB, nvB;
-  u32 never;  // stands in for the alpha string of an idle lane: at distance > 4 from every key and pad
-  u32 pad;    // pads the staged blocks: at distance > 4 from every alpha string
-  int pow2;   // noA > 4: the alpha-beta test is "a & ~k has at most one bit" (no POPC), which pad = 0 never passes
+  int norb;  // orbitals a lane tests: min(noA, nvA)
+  int occ;   // 1: the lane's occupied orbitals (a key's missing bits are counted), 0: its virtual ones (a key's extra bits)
 };
 
 struct LaneHits {  // where a lane's sample keeps its hits in the global buffer
@@ -119,13 +110,12 @@ struct LaneHits {  // where a lane's sample keeps its hits in the global buffer
 
 // what the rarely taken paths of a tile need (kept in local memory; the inner loop never touches it)
 struct TileCtx {
-  BlockWarpSmem *S;
   const u64 *keysB;
   u32 *self_pos, *hits;
   HitRun *my_runs;
   ElocCounters *ctr;
   u64 x;
-  u32 a, sid, hit_cap;
+  u32 sid, hit_cap;
   int run_stride;
 };
 
@@ -161,162 +151,135 @@ __device__ __forceinline__ void emit_hit(const TileCtx &c, LaneHits &h, u32 v) {
   c.hits[h.base + h.fill++] = v;
 }
 
-__device__ __forceinline__ void cp_async4(u32 *smem_dst, const u32 *gsrc) {
+__device__ __forceinline__ void cp_async16(u32 *smem_dst, const u32 *gsrc) {
   const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(gsrc) : "memory");
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-// the queue holds blocks (8 staged keys) that contained a hit: look at each key again and emit the hits.  The lanes
-// stay together: entry i of every lane is examined at the same time, then the hits are emitted bit by bit
-template <bool OWN>
-__device__ __noinline__ LaneHits flush_blocks(const TileCtx &c, u32 qn, LaneHits h) {
-  BlockWarpSmem &S = *c.S;
-  const int lane = threadIdx.x & 31;
-  const u32 a = c.a;
-  const u32 mx = __reduce_max_sync(0xffffffffu, qn);
-  for (u32 i = 0; i < mx; ++i) {
-    u32 m = 0, gpos = 0;
-    if (i < qn) {
-      const u32 j = S.queue[i * 32 + lane];
-      gpos = S.blkpos[j >> 3];
-      const uint4 k0 = *reinterpret_cast<const uint4 *>(&S.stage[j]), k1 = *reinterpret_cast<const uint4 *>(&S.stage[j + 4]);
-      const u32 k[8] = {k0.x, k0.y, k0.z, k0.w, k1.x, k1.y, k1.z, k1.w};
+// The key test.  All alpha strings of the sector have noA bits, so |a ^ k| = 2 |k & ~a| = 2 |a & ~k|: key k is an alpha
+// single of the lane's string a iff exactly one of k's bits lies on a's virtual orbitals (equivalently: exactly one of a's
+// occupied orbitals is missing from k), an alpha double iff two do, and k == a iff none does.  A lane counts that number
+// on the smaller side, K = min(noA, nvA) orbitals, for 32 keys at once: the bit planes of a chunk (planes[o] = bit o of
+// its 32 folded alpha strings) of its K orbitals through a saturating bit-sliced counter.
+// KT: K at compile time (OCC: the occupied side); KT < 0: any K up to kMaxOrbs, side chosen at run time.
+template <int KT, bool OCC>
+struct LaneOrbs {
+  u32 pos[KT >= 0 ? (KT > 0 ? KT : 1) : kMaxOrbs];  // the lane's K orbitals (folded positions)
+  int k;                                             // KT < 0: K
+  u32 flip;                                          // KT < 0: ~0 on the occupied side
+};
+
+template <int KT, bool OCC>
+__device__ __forceinline__ LaneOrbs<KT, OCC> lane_orbs(u32 fa, u32 all_alpha, const BlockGeom &g) {
+  LaneOrbs<KT, OCC> o;
+  o.k = g.norb;
+  o.flip = g.occ ? 0xffffffffu : 0u;
+  u32 s = (KT < 0 ? g.occ != 0 : OCC) ? fa : all_alpha & ~fa;
+  constexpr int kn = KT >= 0 ? KT : kMaxOrbs;
 #pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const u32 d = (u32)__popc(k[u] ^ a);
-        if (OWN) {
-          if (d == 0u) {
-            if (c.keysB[gpos + u] == c.x) c.self_pos[c.sid] = gpos + u;  // the sample itself (checked on the full key)
-          } else if (d == 2u || d == 4u) {
-            m |= 1u << u;
-          }
-        } else if (d == 2u) {
-          m |= 1u << u;
-        }
-      }
-    }
-    while (__any_sync(0xffffffffu, m != 0u)) {
-      if (m) {
-        const int u = __ffs(m) - 1;
-        m &= m - 1u;
-        emit_hit(c, h, (gpos + (u32)u) | (OWN ? kHitOwn : 0u));
-      }
-    }
+  for (int k = 0; k < kn; ++k) {
+    o.pos[k] = (u32)(__ffs(s) - 1) & 31u;  // (an idle lane's string has no bits: any position will do)
+    s &= s - 1u;
   }
-  return h;
+  return o;
 }
 
-// test the staged keys [0, cnt) (cnt a multiple of 16) against the lane's alpha string: 3 instructions per key
-// (XOR, POPC, compare-and-accumulate into a predicate), one queue entry per block of 8 keys with a hit
-// (POW2: a and k have the same number of bits, so they differ in one orbital pair iff a & ~k is a single bit;
-//  v & (v - 1) == 0 also lets k == a through, which the exact test of flush_blocks drops.  ALU / FMA pipes instead
-//  of the quarter-rate POPC pipe: 7.0 instead of 8.8 cycles per key and scheduler, profiles/micro/test_rate.cu)
-__device__ __forceinline__ bool one_pair(u32 a, u32 k) {
-  const u32 v = a & ~k;
-  return (v & (v - 1u)) == 0u;
-}
-
-template <bool OWN, bool POW2>
-__device__ __forceinline__ void test_stage(const TileCtx &c, LaneHits &h, BlockWarpSmem &S, u32 cnt, u32 a) {
-  const int lane = threadIdx.x & 31;
-  const uint4 *st4 = reinterpret_cast<const uint4 *>(S.stage);
-  char *qbase = reinterpret_cast<char *>(&S.queue[lane]);
-  u32 qoff = 0;  // 64 * number of queued entries
-  for (u32 j = 0; j < cnt; j += 16) {
-    const uint4 k0 = st4[(j >> 2)], k1 = st4[(j >> 2) + 1], k2 = st4[(j >> 2) + 2], k3 = st4[(j >> 2) + 3];
-    bool h0, h1;
-    if (OWN) {
-      h0 = (__popc(k0.x ^ a) <= 4) | (__popc(k0.y ^ a) <= 4) | (__popc(k0.z ^ a) <= 4) | (__popc(k0.w ^ a) <= 4) | (__popc(k1.x ^ a) <= 4) |
-           (__popc(k1.y ^ a) <= 4) | (__popc(k1.z ^ a) <= 4) | (__popc(k1.w ^ a) <= 4);
-      h1 = (__popc(k2.x ^ a) <= 4) | (__popc(k2.y ^ a) <= 4) | (__popc(k2.z ^ a) <= 4) | (__popc(k2.w ^ a) <= 4) | (__popc(k3.x ^ a) <= 4) |
-           (__popc(k3.y ^ a) <= 4) | (__popc(k3.z ^ a) <= 4) | (__popc(k3.w ^ a) <= 4);
-    } else if (POW2) {
-      h0 = one_pair(a, k0.x) | one_pair(a, k0.y) | one_pair(a, k0.z) | one_pair(a, k0.w) | one_pair(a, k1.x) | one_pair(a, k1.y) |
-           one_pair(a, k1.z) | one_pair(a, k1.w);
-      h1 = one_pair(a, k2.x) | one_pair(a, k2.y) | one_pair(a, k2.z) | one_pair(a, k2.w) | one_pair(a, k3.x) | one_pair(a, k3.y) |
-           one_pair(a, k3.z) | one_pair(a, k3.w);
-    } else {
-      h0 = (__popc(k0.x ^ a) == 2) | (__popc(k0.y ^ a) == 2) | (__popc(k0.z ^ a) == 2) | (__popc(k0.w ^ a) == 2) | (__popc(k1.x ^ a) == 2) |
-           (__popc(k1.y ^ a) == 2) | (__popc(k1.z ^ a) == 2) | (__popc(k1.w ^ a) == 2);
-      h1 = (__popc(k2.x ^ a) == 2) | (__popc(k2.y ^ a) == 2) | (__popc(k2.z ^ a) == 2) | (__popc(k2.w ^ a) == 2) | (__popc(k3.x ^ a) == 2) |
-           (__popc(k3.y ^ a) == 2) | (__popc(k3.z ^ a) == 2) | (__popc(k3.w ^ a) == 2);
-    }
-    if (h0) {
-      *reinterpret_cast<unsigned short *>(qbase + qoff) = (unsigned short)j;
-      qoff += 64u;
-    }
-    if (h1) {
-      *reinterpret_cast<unsigned short *>(qbase + qoff) = (unsigned short)(j + 8u);
-      qoff += 64u;
-    }
-    if (__any_sync(0xffffffffu, qoff > 64u * (u32)(kQCap - 2))) {
-      h = flush_blocks<OWN>(c, qoff >> 6, h);
-      qoff = 0;
-    }
+// ones / twos / threes: the keys of the staged chunk with at least 1 / 2 / 3 counted orbitals
+template <int KT, bool OCC>
+__device__ __forceinline__ void count_orbs(const u32 *st, const LaneOrbs<KT, OCC> &o, u32 &ones, u32 &twos, u32 &threes) {
+  ones = twos = threes = 0u;
+  constexpr int kn = KT >= 0 ? KT : kMaxOrbs;
+#pragma unroll
+  for (int k = 0; k < kn; ++k) {
+    if (KT < 0 && k >= o.k) break;
+    u32 x = st[o.pos[k]];
+    if (KT < 0) x ^= o.flip;
+    else if (OCC) x = ~x;
+    threes |= twos & x;
+    twos |= ones & x;
+    ones |= x;
   }
-  h = flush_blocks<OWN>(c, qoff >> 6, h);
 }
 
 // Walk the groups [q_lo, q_hi) of the current beta string: S.goff[q_lo .. q_hi] holds the exclusive prefix of their
-// sizes in blocks of 8 keys.  Fill after fill: block descriptors (lanes over groups), copy (8 lanes per block, cp.async),
-// test.
-template <bool OWN>
-__device__ __forceinline__ void walk_groups(TileCtx &c, LaneHits &h, BlockWarpSmem &S, const BlockGeom &g, const u32 *__restrict__ halfB,
-                                            int q_lo, int q_hi, u32 a) {
+// sizes in chunks of 32 keys (chunk c = positions 32c .. 32c + 31 of the beta-grouped copy; a group's first and last
+// chunk are shared with its neighbours and masked).  Fill after fill: chunk descriptors (lanes over groups), copy of
+// their bit planes (8 lanes per chunk, cp.async), test.  Every lane emits its hits in ascending position within a group,
+// the groups in the order of q.  live: ~0 for a lane whose sample has the walk's beta string, else 0.
+template <bool OWN, int KT, bool OCC>
+__device__ __forceinline__ void walk_groups(const TileCtx &c, LaneHits &h, BlockWarpSmem &S, const u32 *__restrict__ planes, int q_lo,
+                                            int q_hi, const LaneOrbs<KT, OCC> &o, u32 live) {
   const int lane = threadIdx.x & 31;
   const u32 total = S.goff[q_hi];
-  for (u32 fb = 0; fb < total; fb += (u32)(kStage / 8)) {
-    const u32 nblk = total - fb < (u32)(kStage / 8) ? total - fb : (u32)(kStage / 8);
+  for (u32 f0 = 0; f0 < total; f0 += (u32)kStageChunks) {
+    const u32 n = total - f0 < (u32)kStageChunks ? total - f0 : (u32)kStageChunks;
     for (int q = q_lo + lane; q < q_hi; q += 32) {
       const u32 g0 = S.goff[q], g1 = S.goff[q + 1];
-      const u32 lo = g0 > fb ? g0 : fb, hi = g1 < fb + nblk ? g1 : fb + nblk;
+      const u32 lo = g0 > f0 ? g0 : f0, hi = g1 < f0 + n ? g1 : f0 + n;
       if (lo < hi) {
         const uint2 r = S.rng[q];
-        for (u32 b = lo; b < hi; ++b) {
-          const u32 first = r.x + 8u * (b - g0), left = r.y - first;
-          S.blkpos[b - fb] = first;
-          S.blkcnt[b - fb] = (unsigned char)(left < 8u ? left : 8u);
+        const u32 c0 = r.x >> 5, c1 = (r.y - 1u) >> 5;
+        for (u32 j = lo; j < hi; ++j) {
+          const u32 cj = c0 + (j - g0);
+          u32 m = 0xffffffffu;
+          if (cj == c0) m &= 0xffffffffu << (r.x & 31u);
+          if (cj == c1) m &= 0xffffffffu >> (31u - ((r.y - 1u) & 31u));
+          S.chunk[j - f0] = make_uint2(cj, m);
         }
       }
     }
     __syncwarp();
-    const u32 nblk2 = (nblk + 1u) & ~1u;  // the test loop takes 16 keys at a time
+    // 8 lanes per chunk, 4 chunks per pass, all passes of the fill in flight (the descriptors are read first: without
+    // that every pass would wait for its own load)
     const u32 sub = (u32)lane & 7u;
-    // 8 lanes per block, 4 blocks per pass, 4 passes in flight (the descriptors come out of shared memory: without the
-    // unrolling every pass would wait for its own two loads)
-    for (u32 b0 = (u32)lane >> 3; b0 < nblk2; b0 += 16) {
-      u32 cnt[4], pos[4];
+    {
+      u32 cj[kStageChunks / 4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const u32 b = b0 + 4u * (u32)u;
-        const bool in = b < nblk;
-        cnt[u] = in ? (u32)S.blkcnt[b] : 0u;
-        pos[u] = in ? S.blkpos[b] : 0u;
+      for (int u = 0; u < kStageChunks / 4; ++u) {
+        const u32 j = ((u32)lane >> 3) + 4u * (u32)u;
+        cj[u] = j < n ? S.chunk[j].x : 0u;
       }
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const u32 b = b0 + 4u * (u32)u;
-        if (b < nblk2) {
-          u32 *dst = &S.stage[8u * b + sub];
-          if (sub < cnt[u]) cp_async4(dst, halfB + pos[u] + sub);
-          else *dst = g.pad;
-        }
+      for (int u = 0; u < kStageChunks / 4; ++u) {
+        const u32 j = ((u32)lane >> 3) + 4u * (u32)u;
+        if (j < n) cp_async16(&S.stage[32u * j + 4u * sub], planes + 32u * (size_t)cj[u] + 4u * sub);
       }
     }
     cp_async_wait_all();
     __syncwarp();
-    c.a = a;
-    if (OWN) test_stage<true, false>(c, h, S, 8u * nblk2, a);
-    else if (g.pow2) test_stage<false, true>(c, h, S, 8u * nblk2, a);
-    else test_stage<false, false>(c, h, S, 8u * nblk2, a);
+    for (u32 j = 0; j < n; ++j) {
+      const uint2 d = S.chunk[j];
+      u32 ones, twos, threes;
+      count_orbs<KT, OCC>(S.stage + 32u * j, o, ones, twos, threes);
+      const u32 keys = d.y & live, base = d.x << 5;
+      u32 m = (OWN ? ones & ~threes : ones & ~twos) & keys;  // own group: singles and doubles; else: singles
+      if (OWN) {
+        u32 self = ~ones & keys;  // the sample itself (checked on the full key)
+        while (self) {
+          const u32 p = base + (u32)(__ffs(self) - 1);
+          self &= self - 1u;
+          if (c.keysB[p] == c.x) c.self_pos[c.sid] = p;
+        }
+      }
+      while (__any_sync(0xffffffffu, m != 0u)) {
+        if (m) {
+          const u32 p = base + (u32)(__ffs(m) - 1);
+          m &= m - 1u;
+          emit_hit(c, h, p | (OWN ? kHitOwn : 0u));
+        }
+      }
+    }
     __syncwarp();
   }
 }
 
+// chunks of 32 keys that the bucket [r.x, r.y) touches
+__device__ __forceinline__ u32 group_chunks(uint2 r) { return r.x == r.y ? 0u : ((r.y - 1u) >> 5) - (r.x >> 5) + 1u; }
+
 // SPLIT: the alpha-beta groups of a tile are split over several warps (see `parts` below); a template parameter so that
 // the whole-tile kernel of large calls carries none of the bookkeeping.
-template <bool SPLIT>
+template <bool SPLIT, int KT, bool OCC>
 __global__ void __launch_bounds__(kBlkWarps * 32)
 eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, const uint2 *__restrict__ tiles, ElocCounters *ctr, GroupView gv,
                   HitRun *__restrict__ runs, u32 *__restrict__ run_cnt, int run_stride, u32 *__restrict__ hits, u32 *__restrict__ self_pos,
@@ -340,9 +303,11 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
   }
   const u32 runs_per_part = (u32)run_stride / parts;
   const u32 nitems = ntiles * parts;
-  const u32 *__restrict__ halfB = gv.half[0];
+  const u32 *__restrict__ planes = gv.planes;
   const u32 *__restrict__ halfA = gv.half[1];
-  const u32 all_beta = fold_beta(g.sorb >= 64 ? ~0ull : ((1ull << g.sorb) - 1ull));
+  const u64 all_orbs = g.sorb >= 64 ? ~0ull : ((1ull << g.sorb) - 1ull);
+  const u32 all_alpha = fold_alpha(all_orbs);
+  const u32 all_beta = fold_beta(all_orbs);
   for (;;) {
     u32 t = 0;
     if (lane == 0) t = atomicAdd(&ctr->tile_next, 1u);
@@ -355,8 +320,8 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
     const u32 sid = active ? slots[tile.x + lane] : 0u;
     const u64 x = active ? bra[sid] : 0ull;
     const u32 fa = fold_alpha(x), fb = fold_beta(x);
+    const LaneOrbs<KT, OCC> orbs = lane_orbs<KT, OCC>(fa, all_alpha, g);
     TileCtx c;
-    c.S = &S;
     c.keysB = gv.keys[0];
     c.self_pos = self_pos;
     c.hits = hits;
@@ -375,7 +340,7 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
       const u32 fbL = __shfl_sync(0xffffffffu, fb, leader);
       const bool mine = active && fb == fbL;
       remaining &= ~__ballot_sync(0xffffffffu, mine);
-      const u32 a = mine ? fa : g.never;
+      const u32 live = mine ? 0xffffffffu : 0u;
       // ---- the groups of this beta string: positions of its occupied / virtual orbitals, then one bucket per single ------
       __syncwarp();
       {
@@ -398,18 +363,17 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
       __syncwarp();
       // the own group first (other acceptance test): the keys that carry the tile's beta string itself
       if (lane == 0) {
-        const uint2 r = S.rng[sB];
         S.goff[sB] = 0u;
-        S.goff[sB + 1] = (r.y - r.x + 7u) >> 3;
+        S.goff[sB + 1] = group_chunks(S.rng[sB]);
       }
       __syncwarp();
-      if (part == 0u) walk_groups<true>(c, h, S, g, halfB, sB, sB + 1, a);
+      if (part == 0u) walk_groups<true>(c, h, S, planes, sB, sB + 1, orbs, live);
       // two singles whose strings share a bucket: the folded test cannot tell them apart, so the bucket is walked for one
       // of them only -- the one with the SMALLEST group number, so that every part of a split tile drops the same ones.
-      // Buckets are told apart by their first position; the set lives in the (now idle) hit queue, the smallest group number
-      // of every bucket in the (now idle) stage buffer, a group's slot of the set in goff (recomputed below)
-      u32 *dupset = reinterpret_cast<u32 *>(S.queue);
-      u32 *minq = S.stage;
+      // Buckets are told apart by their first position; the set and the smallest group number of every bucket live in the
+      // (now idle) stage buffer, a group's slot of the set in goff (recomputed below)
+      u32 *dupset = S.stage;
+      u32 *minq = S.stage + kDupSet;
       for (int i = lane; i < kDupSet; i += 32) {
         dupset[i] = 0xffffffffu;
         minq[i] = 0xffffffffu;
@@ -433,16 +397,13 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
         if (r.x != r.y && minq[S.goff[q]] != (u32)q) S.rng[q] = make_uint2(0u, 0u);
       }
       __syncwarp();
-      // first block of every group: exclusive prefix over the groups' sizes in blocks of 8
+      // first chunk of every group: exclusive prefix over the groups' sizes in chunks
       {
         u32 running = 0;
         for (int q0 = 0; q0 < sB; q0 += 32) {
           const int q = q0 + lane;
           u32 nb = 0;
-          if (q >= q_part_lo && q < q_part_hi) {  // (the buckets of the other parts' groups count as empty here)
-            const uint2 r = S.rng[q];
-            nb = (r.y - r.x + 7u) >> 3;
-          }
+          if (q >= q_part_lo && q < q_part_hi) nb = group_chunks(S.rng[q]);  // (the other parts' groups count as empty)
           u32 incl = nb;
 #pragma unroll
           for (int o = 1; o < 32; o <<= 1) {
@@ -455,7 +416,7 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
         if (lane == 0) S.goff[sB] = running;
       }
       __syncwarp();
-      walk_groups<false>(c, h, S, g, halfB, 0, sB, a);
+      walk_groups<false>(c, h, S, planes, 0, sB, orbs, live);
     }
     // ---- every sample's own-alpha group (beta singles, beta-beta doubles): the group depends on the sample, so every lane
     // walks ITS bucket of the alpha-grouped copy, four independent loads in flight (a lane reads consecutive words: its lines
@@ -507,6 +468,17 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
 }
 
 // ---- host side --------------------------------------------------------------------------------------------------------
+using BlockKernel = decltype(&eloc_block_kernel<false, -1, false>);
+
+// K at compile time for the benchmarked Fe2S2 sector (5 virtual alpha orbitals) and the geometries the tests cover
+template <bool SPLIT>
+static BlockKernel block_kernel(const BlockGeom &bg) {
+  if (bg.norb == 5) return bg.occ ? eloc_block_kernel<SPLIT, 5, true> : eloc_block_kernel<SPLIT, 5, false>;
+  if (bg.norb == 6 && !bg.occ) return eloc_block_kernel<SPLIT, 6, false>;
+  if (bg.norb == 8 && bg.occ) return eloc_block_kernel<SPLIT, 8, true>;
+  return eloc_block_kernel<SPLIT, -1, false>;
+}
+
 struct BlockLayout {
   u32 log2_buckets;
   long long bcnt, bbase, slots, tiles, total;
@@ -556,10 +528,8 @@ int launch_eloc_block(const u64 *bra, long long n, const GroupView &gv, char *bl
   bg.noA = g.noA;
   bg.noB = g.noB;
   bg.nvB = g.nvB;
-  // idle lanes and pads must never pass a test, against real strings (noA bits) and against each other
-  bg.never = g.noA > 4 ? 0xffffffffu : 0x0000ffffu;  // distance >= 16 - noA >= 12 from every key, >= 16 from the pad
-  bg.pad = g.noA > 4 ? 0u : 0xffffffffu;             // distance noA resp. 32 - noA from every alpha string
-  bg.pow2 = g.noA > 4;
+  bg.occ = g.noA < g.nvA;
+  bg.norb = bg.occ ? g.noA : g.nvA;
   const size_t smem = sizeof(BlockWarpSmem) * kBlkWarps;
   long long ctas = (n + 32 * kBlkWarps - 1) / (32 * kBlkWarps);
   const long long cap = 148LL * (long long)((227 * 1024) / (sizeof(BlockWarpSmem) * kBlkWarps + 1024));
@@ -567,7 +537,7 @@ int launch_eloc_block(const u64 *bra, long long n, const GroupView &gv, char *bl
   // fewer than ~2 tiles (of ~26 samples) per resident warp: split the tiles (the knob block_parts forces 1, 2 or 4 parts)
   const int forced = eloc_tuning().block_parts;
   const bool split = forced ? forced > 1 : n < 2 * 26 * ctas * kBlkWarps;
-  auto kern = split ? eloc_block_kernel<true> : eloc_block_kernel<false>;
+  const BlockKernel kern = split ? block_kernel<true>(bg) : block_kernel<false>(bg);
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return check_launch("eloc_block_kernel smem opt-in");
   kern<<<(unsigned)ctas, kBlkWarps * 32, smem, st>>>(bra, slots, tiles, ctr, gv, runs, run_cnt, run_stride, hits, self_pos, hit_cap, bg,

@@ -4,7 +4,8 @@
 //               string); adjacent equal keys raise has_dup;
 //   2. sort   : one stable radix sort per grouping of (bucket id, row) over log2(buckets) bits
 //               (cub onesweep) -- rows inside a bucket stay ascending;
-//   3. finish : gather the keys into bucket order and write the bucket boundaries.
+//   3. finish : gather the keys into bucket order and write the bucket boundaries (and, L = 1, the bit planes of the
+//               beta-grouped copy's folded alpha strings).
 #include <mutex>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -37,6 +38,8 @@ GroupLayout group_layout(long long N, int L) {
   }
   l.pos_off = o;
   o = up(o + N * 4);
+  l.planes_off = o;
+  if (L == 1) o = up(o + (N + 31) / 32 * 128);
   l.scratch_off = o;
   for (int g = 0; g < 2; ++g)
     for (int k = 0; k < 2; ++k) {
@@ -68,6 +71,7 @@ GroupView group_view(const void *ws, long long N, int L) {
     v.half[g] = L == 1 ? reinterpret_cast<const u32 *>(b + l.half_off[g]) : nullptr;
   }
   v.pos = reinterpret_cast<const u32 *>(b + l.pos_off);
+  v.planes = L == 1 ? reinterpret_cast<const u32 *>(b + l.planes_off) : nullptr;
   v.shift = 32u - l.log2_buckets;
   return v;
 }
@@ -96,10 +100,22 @@ __global__ void __launch_bounds__(256)
 group_finish_kernel(const u64 *__restrict__ key, long long N, u32 log2_buckets, const u32 *__restrict__ bktB,
                     const u32 *__restrict__ bktA, const u32 *__restrict__ rowsB, const u32 *__restrict__ rowsA, u64 *__restrict__ keysB,
                     u64 *__restrict__ keysA, u32 *__restrict__ startB, u32 *__restrict__ startA, u32 *__restrict__ halfB,
-                    u32 *__restrict__ halfA, u32 *__restrict__ posB) {
+                    u32 *__restrict__ halfA, u32 *__restrict__ posB, u32 *__restrict__ planes) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= N) return;
   const bool ga = blockIdx.y != 0;
+  if (L == 1 && !ga && (i & ~31LL) < N) {
+    // the folded alpha strings of the warp's 32 positions bit-transposed: one ballot per bit, lane o keeps ballot o
+    // (blocks are whole warps, so all 32 lanes are here; the positions past N count as empty strings)
+    const u32 fa = i < N ? fold_alpha(key[rowsB[i]]) : 0u;
+    u32 plane = 0;
+#pragma unroll
+    for (int o = 0; o < 32; ++o) {
+      const u32 b = __ballot_sync(0xffffffffu, (fa >> o) & 1u);
+      if ((threadIdx.x & 31) == o) plane = b;
+    }
+    planes[i] = plane;  // = planes[(i / 32) * 32 + lane]
+  }
+  if (i >= N) return;
   const u32 *bkt = ga ? bktA : bktB;
   const u32 *rows = ga ? rowsA : rowsB;
   u64 *keys = ga ? keysA : keysB;
@@ -189,6 +205,7 @@ int launch_group_build(const u64 *key, long long N, int L, void *ws, long long w
   u32 *iota = reinterpret_cast<u32 *>(b + l.iota_off);
   u32 *half[2] = {reinterpret_cast<u32 *>(b + l.half_off[0]), reinterpret_cast<u32 *>(b + l.half_off[1])};
   u32 *posB = reinterpret_cast<u32 *>(b + l.pos_off);
+  u32 *planes = reinterpret_cast<u32 *>(b + l.planes_off);
   if (cudaMemsetAsync(hdr, 0, sizeof(GroupHeader), st) != cudaSuccess) return check_launch("group header memset");
   if (N == 0) {
     group_empty_kernel<<<148, 256, 0, st>>>(hdr, l.log2_buckets, start[0], start[1]);
@@ -221,7 +238,7 @@ int launch_group_build(const u64 *key, long long N, int L, void *ws, long long w
   const dim3 grid(blocks, 2);
 #define PYNQS_FINISH(LL)                                                                                                           \
   group_finish_kernel<LL><<<grid, 256, 0, st>>>(key, N, l.log2_buckets, bkt[0][1], bkt[1][1], rows[0], rows[1], keys[0], keys[1], \
-                                                start[0], start[1], half[0], half[1], posB)
+                                                start[0], start[1], half[0], half[1], posB, planes)
   switch (L) {
     case 1: PYNQS_FINISH(1); break;
     case 2: PYNQS_FINISH(2); break;

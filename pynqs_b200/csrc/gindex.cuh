@@ -38,7 +38,7 @@ static_assert(sizeof(GroupHeader) == 256, "header is 256 bytes");
 
 struct GroupLayout {
   u32 log2_buckets;
-  long long start_off[2], keys_off[2], rows_off[2], half_off[2], pos_off, scratch_off, total;
+  long long start_off[2], keys_off[2], rows_off[2], half_off[2], pos_off, planes_off, scratch_off, total;
   long long bkt_off[2][2], iota_off;  // build scratch: bucket ids (in / out per grouping), identity rows
   long long cub_off;
   size_t cub_bytes;
@@ -57,6 +57,7 @@ struct GroupView {
   const u32 *rows[2];
   const u32 *half[2];  // L = 1 only: [0] folded alpha strings in B order, [1] folded beta strings in A order
   const u32 *pos;      // position of every row of the sorted table in the beta-grouped copy (inverse of rows[0])
+  const u32 *planes;   // L = 1 only: half[0] bit-transposed, planes[c * 32 + o] = bit o of the keys c * 32 .. c * 32 + 31
   u32 shift;  // 32 - log2_buckets
 };
 
