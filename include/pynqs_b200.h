@@ -179,6 +179,20 @@ int pynqs_hamiltonian_emit(const uint8_t *bra, int64_t n, const double *h1e, con
 int pynqs_csr_spmm(const int64_t *crow, const int64_t *col, const double *val, int64_t n, int64_t N, const double *X, int64_t ldx, int k,
                    double *Y, int64_t ldy, void *stream);
 
+/* Additive op: Y = S^2 X over the sorted key table, Y[i, c] = sum over j < N of <bra_i|S^2|key_j> X[j, c], for row-major
+ * blocks X double[N, k] (row stride ldx) and Y double[n, k] (row stride ldy), 1 <= k <= 8; wider blocks go through in column
+ * slices as for pynqs_csr_spmm.  Orbital i has alpha at bit 2i and beta at bit 2i + 1.  With A / B the alpha-only / beta-only
+ * orbitals of x and Sz = (n_alpha - n_beta) / 2, taken from x's own bits:  <x|S^2|x> = |B| + Sz (Sz + 1), counted when x is
+ * in the table;  <x|S^2|x ^ (3 << 2p) ^ (3 << 2q)> = +1 for p in A, q in B, counted when that spin exchange is in the table.
+ * A table with duplicate keys gives the column the classic binary search lands on.  key / group_ws as for
+ * pynqs_eloc_sample_space (N < 2^31).  Deterministic: row i is summed in one fixed order (the diagonal, then the partners in
+ * ascending (p, q)); no scratch, no host synchronisation.  PYNQS_EVALUE, before anything touches the device, for an odd sorb
+ * or one outside (0, PYNQS_MAX_SORB] (the ONV width is (sorb - 1) / 64 + 1 words), n < 0, N < 0 or >= 2^31, k outside
+ * [1, 8], ldx < k, ldy < k, or a NULL bra / Y (n > 0) or key / group_ws / X (n > 0 and N > 0).  n == 0 does nothing;
+ * N == 0 launches no kernel and clears Y. */
+int pynqs_spin_square_apply(const uint8_t *bra, int64_t n, int sorb, const uint8_t *key, int64_t N, const void *group_ws,
+                            const double *X, int64_t ldx, int k, double *Y, int64_t ldy, void *stream);
+
 /* ---- REDUCE method (vmc/energy/eloc.py:257-297, additive) -----------------------------------------
  * The reference materialises comb [n, M, 8L] and Hmat [n, M] and keeps torch.where(|Hmat| >= eps).  These
  * entry points return the kept rows only, in the same (ascending flat index s * M + m) order:

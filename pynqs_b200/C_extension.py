@@ -682,20 +682,10 @@ def csr_matmul(crow: Tensor, col: Tensor, val: Tensor, X: Tensor, N: int) -> Ten
         raise ValueError("crow must be 1-D [n + 1], col and val 1-D of the same length")
     for t, nm in ((crow, "crow"), (col, "col"), (val, "val")):
         _contig(t, nm)
-    if X.dtype not in (torch.float64, torch.complex128):
-        raise ValueError(f"X must be float64 or complex128, got {X.dtype}")
     N = int(N)
-    if X.dim() not in (1, 2) or X.size(0) != N:
-        raise ValueError(f"X must be [N] or [N, k] with N = {N}, got {tuple(X.shape)}")
     n = crow.numel() - 1
-    Xr = X.unsqueeze(1) if X.dim() == 1 else X
-    if (Xr.size(1) > 1 and Xr.stride(1) != 1) or (N > 1 and Xr.stride(0) < Xr.size(1)):
-        Xr = Xr.contiguous()  # the kernel reads rows of adjacent columns, rows apart by ldx >= k
-    if X.is_complex():
-        Xr = torch.view_as_real(Xr.resolve_conj())
-        Xr = Xr.as_strided((N, 2 * Xr.size(1)), (Xr.stride(0), 1))  # [N, k, 2] with adjacent columns -> real [N, 2k]
+    Xr, ldx = _real_block(X, N)
     kk = Xr.size(1)
-    ldx = Xr.stride(0) if N > 1 else kk  # a single row's stride is not meaningful
     work = n > 0 and N > 0 and col.numel() > 0 and kk > 0
     Y = (torch.empty if work else torch.zeros)((n, kk), dtype=torch.float64, device=dev)
     if work:
@@ -706,9 +696,69 @@ def csr_matmul(crow: Tensor, col: Tensor, val: Tensor, X: Tensor, N: int) -> Ten
                 _lib.check(lib.pynqs_csr_spmm(vp(crow.data_ptr()), vp(col.data_ptr()), vp(val.data_ptr()), i64(n), i64(N),
                                               vp(Xr.data_ptr() + 8 * c0), i64(ldx), int(k), vp(Y.data_ptr() + 8 * c0), i64(kk),
                                               _stream(dev)))
+    return _from_real_block(Y, X)
+
+
+def _real_block(X: Tensor, N: int) -> Tuple[Tensor, int]:
+    """X float64 / complex128 [N] or [N, k] as the real row-major block the block kernels read: (Xr float64 [N, k'], ldx),
+    k' = k for a real X and 2k for a complex one (its torch.view_as_real view, real and imaginary parts as adjacent
+    columns).  Rows may be strided; columns that are not adjacent are copied."""
+    if X.dtype not in (torch.float64, torch.complex128):
+        raise ValueError(f"X must be float64 or complex128, got {X.dtype}")
+    if X.dim() not in (1, 2) or X.size(0) != N:
+        raise ValueError(f"X must be [N] or [N, k] with N = {N}, got {tuple(X.shape)}")
+    Xr = X.unsqueeze(1) if X.dim() == 1 else X
+    if (Xr.size(1) > 1 and Xr.stride(1) != 1) or (N > 1 and Xr.stride(0) < Xr.size(1)):
+        Xr = Xr.contiguous()  # the kernel reads rows of adjacent columns, rows apart by ldx >= k
     if X.is_complex():
-        Y = torch.view_as_complex(Y.view(n, kk // 2, 2))
+        Xr = torch.view_as_real(Xr.resolve_conj())
+        Xr = Xr.as_strided((N, 2 * Xr.size(1)), (Xr.stride(0), 1))  # [N, k, 2] with adjacent columns -> real [N, 2k]
+    return Xr, (Xr.stride(0) if N > 1 else Xr.size(1))  # a single row's stride is not meaningful
+
+
+def _from_real_block(Y: Tensor, X: Tensor) -> Tensor:
+    """The real result block Y [n, k'] of a kernel that read _real_block(X) in X's dtype and shape."""
+    n = Y.size(0)
+    if X.is_complex():
+        Y = torch.view_as_complex(Y.view(n, Y.size(1) // 2, 2))
     return Y.view(n) if X.dim() == 1 else Y
+
+
+def spin_square_matmul(bra: Tensor, sorb: int, bra_key: Tensor, X: Tensor, group_index: GroupIndex | None = None) -> Tensor:
+    """Y = S^2 X over the sorted key table: Y[i] = sum over j of <bra_i|S^2|bra_key_j> X[j] (pynqs_spin_square_apply).  The
+    diagonal |B| + Sz (Sz + 1) counts when bra_i is in the table; the +1 of each spin exchange of bra_i (an alpha-only and a
+    beta-only orbital that swap their spins) counts when that determinant is in the table.  Sz comes from each row's own
+    bits.  With bra = bra_key this is S^2 restricted to the sample set, in the table's row order.
+
+    X: float64 or complex128, [N] or [N, k] of any k, handled as csr_matmul handles it; Y has X's dtype and shape with n
+    rows.  group_index: the table's GroupIndex (WavefunctionLUT.group_index), built and cached when not given.
+    Deterministic (identical bits on every call); no host synchronisation."""
+    dev = _need_cuda(bra, bra_key, X)
+    for t, nm in ((bra, "bra"), (bra_key, "bra_key")):
+        _contig(t, nm)
+    if bra.dim() != 2 or bra_key.dim() != 2:
+        raise ValueError("bra and bra_key must be 2-D [rows, 8L]")
+    L = _check_width(bra, sorb, "bra")
+    if _onv_words(bra_key, "bra_key") != L:
+        raise ValueError("bra and bra_key widths differ")
+    n, N = bra.size(0), bra_key.size(0)
+    Xr, ldx = _real_block(X, N)
+    kk = Xr.size(1)
+    work = n > 0 and N > 0 and kk > 0
+    Y = (torch.empty if work else torch.zeros)((n, kk), dtype=torch.float64, device=dev)
+    if work:
+        if group_index is None:
+            group_index = _cached_group(bra_key)
+        if group_index.N != N or group_index.L != L or group_index.key_ptr != bra_key.data_ptr():
+            raise ValueError("group_index was built for another key table")
+        lib = _lib.load()
+        with torch.cuda.device(dev):
+            for c0 in range(0, kk, 8):
+                k = min(8, kk - c0)
+                _lib.check(lib.pynqs_spin_square_apply(vp(bra.data_ptr()), i64(n), int(sorb), vp(bra_key.data_ptr()), i64(N),
+                                                       vp(group_index.workspace.data_ptr()), vp(Xr.data_ptr() + 8 * c0), i64(ldx),
+                                                       int(k), vp(Y.data_ptr() + 8 * c0), i64(kk), _stream(dev)))
+    return _from_real_block(Y, X)
 
 
 def lookup_compact(idx_array: Tensor, mask: Tensor, wf_value: Tensor) -> Tuple[Tensor, Tensor, Tensor]:

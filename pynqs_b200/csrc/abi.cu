@@ -83,6 +83,8 @@ int launch_onv_to_tensor(const u64 *, void *, int, long long, int, cudaStream_t)
 int launch_tensor_to_onv(const unsigned char *, unsigned char *, long long, int, cudaStream_t);
 int launch_csr_spmm(const long long *, const long long *, const double *, long long, const double *, long long, int, double *, long long,
                     cudaStream_t);
+int launch_spin_square(const u64 *, long long, int, const u64 *, long long, const void *, const double *, long long, int, double *,
+                       long long, cudaStream_t);
 
 static int check_geometry(int sorb, int nele, int noA, int noB) {
   if (sorb <= 0 || sorb > PYNQS_MAX_SORB) {
@@ -454,6 +456,31 @@ int pynqs_csr_spmm(const int64_t *crow, const int64_t *col, const double *val, i
   if (n == 0) return 0;
   return launch_csr_spmm(reinterpret_cast<const long long *>(crow), reinterpret_cast<const long long *>(col), val, n, X, ldx, k, Y, ldy,
                          (cudaStream_t)stream);
+}
+
+int pynqs_spin_square_apply(const uint8_t *bra, int64_t n, int sorb, const uint8_t *key, int64_t N, const void *group_ws, const double *X,
+                            int64_t ldx, int k, double *Y, int64_t ldy, void *stream) {
+  if (sorb <= 0 || sorb > PYNQS_MAX_SORB || (sorb & 1)) {
+    set_error("spin_square_apply: sorb = %d must be even and in (0, %d]", sorb, PYNQS_MAX_SORB);
+    return PYNQS_EVALUE;
+  }
+  if (n < 0 || N < 0 || N >= (1LL << 31) || k < 1 || k > 8 || ldx < k || ldy < k) {
+    set_error("spin_square_apply: bad n = %lld, N = %lld, k = %d, ldx = %lld or ldy = %lld (N < 2^31, k in [1, 8], ld >= k)",
+              (long long)n, (long long)N, k, (long long)ldx, (long long)ldy);
+    return PYNQS_EVALUE;
+  }
+  if (n > 0 && (bra == nullptr || Y == nullptr || (N > 0 && (key == nullptr || group_ws == nullptr || X == nullptr)))) {
+    set_error("spin_square_apply: null pointer (bra / Y for n > 0, key / group_ws / X as well for N > 0)");
+    return PYNQS_EVALUE;
+  }
+  if (n == 0) return 0;
+  if (N == 0) {  // no partner and no diagonal is in an empty table: Y = 0, without a kernel
+    if (cudaMemset2DAsync(Y, 8 * (size_t)ldy, 0, 8 * (size_t)k, (size_t)n, (cudaStream_t)stream) != cudaSuccess)
+      return check_launch("spin_square_apply: memset of Y");
+    return 0;
+  }
+  return launch_spin_square(reinterpret_cast<const u64 *>(bra), n, (sorb - 1) / 64 + 1, reinterpret_cast<const u64 *>(key), N, group_ws, X,
+                            ldx, k, Y, ldy, (cudaStream_t)stream);
 }
 
 int64_t pynqs_reduce_scratch_bytes(int64_t n) { return reduce_scratch_bytes(n); }

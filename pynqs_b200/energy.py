@@ -64,7 +64,7 @@ def sample_space_hamiltonian(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: Wavefu
 
 def sample_space_ground_state(WF_LUT: WavefunctionLUT, h1e: Tensor, h2e: Tensor, sorb: int, nele: int, noa: int, nob: int,
                               nroots: int = 1, *, H: "Tensor | None" = None, guess: "Tensor | None" = None, tol: float = 1e-8,
-                              max_iter: int = 200) -> Tuple[Tensor, Tensor, dict]:
+                              max_iter: int = 200, spin_shift: float = 0.0, ss: "float | None" = None) -> Tuple[Tensor, Tensor, dict]:
     """The lowest `nroots` eigenpairs of the square sample-space Hamiltonian over the determinants of WF_LUT.bra_key: the
     variational energies within the sample set and their CI coefficients.  Block Davidson (pynqs_b200.davidson) with
     H X = C_extension.csr_matmul on the device CSR matrix and the diagonal <x|H|x> as preconditioner.
@@ -72,9 +72,21 @@ def sample_space_ground_state(WF_LUT: WavefunctionLUT, h1e: Tensor, h2e: Tensor,
     H: sample_space_hamiltonian(WF_LUT.bra_key, ...) (built when not given; pass it to reuse it).  guess: [N] or [N, b] start
     vectors, e.g. the real part of a VMC psi (default: unit vectors on the nroots lowest diagonal entries, ties broken by
     table row).  Returns (energies [nroots] ascending, electronic like eloc; coeffs [N, nroots] orthonormal, rows in the
-    order of WF_LUT.bra_key; info of davidson: iterations, products, residual_norms, converged)."""
+    order of WF_LUT.bra_key; info of davidson: iterations, products, residual_norms, converged).
+
+    spin_shift > 0 targets a spin state, as PySCF's fix_spin_(shift, ss) does: the solver works on H + spin_shift S^2
+    (ss = None: the lowest spins come first) or on H + spin_shift (S^2 - ss)^2 (the states with <S^2> = ss come first), with
+    S^2 restricted to the sample set (C_extension.spin_square_matmul) and the exact diagonal of that operator as
+    preconditioner.  The roots are then ordered by the penalised eigenvalues, `energies` are <c|H|c> of the converged
+    vectors, and info["s2"] holds <c|S^2|c> of each root.  The penalty pins a spin only where the sample set is closed under
+    spin exchanges (the CI space is; a random sample set is not, and its restricted S^2 has no exact spin eigenstates).
+    The iterations grow with spin_shift, because the diagonal preconditioner does not see the penalty's spin-exchange
+    couplings: take the smallest shift that lifts the other sectors above the wanted state.  spin_shift = 0 (the default)
+    solves H alone."""
     keys = WF_LUT.bra_key
     N = keys.size(0)
+    if spin_shift < 0 or (ss is not None and spin_shift == 0):
+        raise ValueError(f"spin_shift = {spin_shift} must be >= 0, and > 0 when ss is given")
     if H is None:
         H = sample_space_hamiltonian(keys, h1e, h2e, WF_LUT, sorb, nele, noa, nob)
     if H.layout != torch.sparse_csr or tuple(H.shape) != (N, N):
@@ -82,7 +94,70 @@ def sample_space_ground_state(WF_LUT: WavefunctionLUT, h1e: Tensor, h2e: Tensor,
     crow, col, val = H.crow_indices(), H.col_indices(), H.values()
     # <x|H|x> from the 3-D form: one ket per bra, bit-identical to the CSR diagonal, nothing of size nnz
     diag = ops.get_hij_torch(keys, keys.view(N, 1, keys.size(1)), h1e, h2e, sorb, nele).view(N)
-    return davidson(lambda V: ops.csr_matmul(crow, col, val, V, N), diag, nroots, guess=guess, tol=tol, max_iter=max_iter)
+    if spin_shift == 0:
+        return davidson(lambda V: ops.csr_matmul(crow, col, val, V, N), diag, nroots, guess=guess, tol=tol, max_iter=max_iter)
+
+    def h_apply(V: Tensor) -> Tensor:
+        return ops.csr_matmul(crow, col, val, V, N)
+
+    def s2_apply(V: Tensor) -> Tensor:
+        return ops.spin_square_matmul(keys, sorb, keys, V, WF_LUT.group_index)
+
+    d = _spin_diagonal(keys)  # every key is in its own table: the restricted S^2 has d on its diagonal
+    if ss is None:
+        def apply(V: Tensor) -> Tensor:
+            return h_apply(V) + spin_shift * s2_apply(V)
+
+        pdiag = diag + spin_shift * d
+    else:
+        def apply(V: Tensor) -> Tensor:
+            W = s2_apply(V) - ss * V
+            return h_apply(V) + spin_shift * (s2_apply(W) - ss * W)
+
+        # diagonal of (S^2 - ss)^2: (d_i - ss)^2 + m_i, m_i = the in-table partners of row i, each an element +1;
+        # S^2 applied to ones gives d_i + m_i
+        m = s2_apply(torch.ones(N, dtype=torch.float64, device=keys.device)) - d
+        pdiag = diag + spin_shift * ((d - ss) ** 2 + m)
+    _, C, info = davidson(apply, pdiag, nroots, guess=guess, tol=tol, max_iter=max_iter)
+    norm = (C * C).sum(0)
+    info["s2"] = ((C * s2_apply(C)).sum(0) / norm).tolist()
+    return (C * h_apply(C)).sum(0) / norm, C, info
+
+
+def _spin_diagonal(x: Tensor) -> Tensor:
+    """<x|S^2|x> = |B| + Sz (Sz + 1) of every ONV row of x (uint8 [n, 8L]), float64 [n]: B = the beta-only orbitals,
+    Sz = (n_alpha - n_beta) / 2 (alpha on the even bits, beta on the odd ones)."""
+    pc = torch.tensor([bin(v).count("1") for v in range(256)], dtype=torch.int64, device=x.device)
+    b = x.long()
+    alpha, beta = b & 0x55, (b >> 1) & 0x55  # the orbitals of each byte, alpha- and beta-occupied
+    na, nb, nB = pc[alpha].sum(1), pc[beta].sum(1), pc[beta & ~alpha].sum(1)
+    sz2 = (na - nb).to(torch.float64)
+    return nB.to(torch.float64) + 0.25 * sz2 * (sz2 + 2.0)
+
+
+def local_spin_square(x: Tensor, WF_LUT: WavefunctionLUT, sorb: int) -> Tuple[Tensor, Tensor]:
+    """The local spin of every sample, S^2_loc(x) = (S^2 psi)(x) / psi(x) with psi = WF_LUT.wf_value over the table (the
+    sample-space convention of local_energy_sample_space: spin exchanges of x that are not in the table count as psi = 0).
+    Returns (s2loc [n], psi_x [n]) in psi's dtype (float64 or complex128); the |psi|^2-weighted mean of s2loc over the table
+    is <S^2> of psi (spin_square).  A sample that is not in the table gets psi_x = 0 and s2loc = NaN, as
+    local_energy_sample_space gives it psi_x = 0 and E_loc = 0/0 = NaN; so does a sample whose table value is 0."""
+    N = WF_LUT.bra_key.size(0)
+    s2psi = ops.spin_square_matmul(x, sorb, WF_LUT.bra_key, WF_LUT.wf_value, WF_LUT.group_index if N > 0 else None)
+    found, _, value = WF_LUT.lookup(x)
+    psi_x = torch.zeros_like(s2psi)
+    psi_x[found] = value
+    nan = complex(float("nan"), float("nan")) if s2psi.is_complex() else float("nan")
+    return torch.where(psi_x == 0, torch.full_like(s2psi, nan), s2psi / psi_x), psi_x
+
+
+def spin_square(WF_LUT: WavefunctionLUT, C: Tensor, sorb: int) -> Tensor:
+    """<S^2> = Re(c^H S^2 c) / (c^H c) of every column c of C (float64 or complex128, [N] or [N, k], rows in the order of
+    WF_LUT.bra_key: Davidson coefficients, or WF_LUT.wf_value), with S^2 restricted to the table.  Returns float64 [k]
+    ([1] for a 1-D C)."""
+    keys = WF_LUT.bra_key
+    C = C.unsqueeze(1) if C.dim() == 1 else C
+    S2C = ops.spin_square_matmul(keys, sorb, keys, C, WF_LUT.group_index)
+    return (C.conj() * S2C).sum(0).real / (C.conj() * C).sum(0).real
 
 
 def local_energy_three_call(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: WavefunctionLUT, sorb: int, nele: int,
