@@ -66,14 +66,15 @@ int launch_scan_batch(const u64 *bra, long long nb, const GroupView &gv, char *s
 int launch_diag_f64(const u64 *bra, const double *h1e, const double *h2e, double *out, long long n, long long stride, int L, int sorb,
                     int nele, cudaStream_t st);
 
-// One hit of sample x decoded (hamiltonian.cu): the key y it points to, y's row of the sorted table, and the class of the pair --
-// 1 single, 2 double, 0 nothing (on the folded route a key that passed the 32-bit test but is not connected to x).
+// One hit of sample x decoded (the evaluation kernels of eloc_scan.cu, hamiltonian.cu): the key y it points to, y's row of the
+// sorted table, and the class of the pair -- 1 single, 2 double, 0 nothing (on the folded route a key that passed the 32-bit
+// test but is not connected to x; row is then not loaded).  It has no warp-wide operation, and every lane returns from it:
+// the callers' ballots that follow need the whole warp.
 template <int L, bool HALF>
 __device__ __forceinline__ int decode_hit(const GroupView &gv, const Onv<L> &x, u32 h, Onv<L> &y, u32 &row) {
   const bool grouping = (h & kHitA) != 0u;
   const u32 pos = HALF ? (h & kHitPos) : (h & ~kHitA);
   y = load_onv<L>((grouping ? gv.keys[1] : gv.keys[0]) + (size_t)pos * L);
-  row = __ldg((grouping ? gv.rows[1] : gv.rows[0]) + pos);
   if (HALF) {  // the scan tested one folded string only: class of the full key vs the scan it came from
     const u64 d = y.w[0] ^ x.w[0];
     const int na = __popcll(d & kEven), nb = __popcll(d & kOdd);
@@ -81,7 +82,50 @@ __device__ __forceinline__ int decode_hit(const GroupView &gv, const Onv<L> &x, 
     const bool ok = (h & kHitOwn) ? ((fixed == 0) & ((moved == 2) | (moved == 4))) : ((na == 2) & (nb == 2));
     if (!ok) return 0;
   }
+  row = __ldg((grouping ? gv.rows[1] : gv.rows[0]) + pos);
   return excitation_class<L>(x, y);
+}
+
+// <x|H|y> of lane src's single excitation x -> y, evaluated by the whole warp (every lane passes the same x; every lane gets
+// the element).  The warp's orbital lists of x are built at the first single of the sample; have_lists remembers that.
+// The callers walk their singles (rare) with a ballot and use the element inside that loop.  (A helper that returned each
+// lane's element after the loop kept one more value live through it: ptxas for sm_100a then gave eloc_eval_kernel<1, false, *>
+// 60 / 64 bytes of spill stores / loads instead of 48 / 48 at its 40-register bound.)
+template <int L>
+__device__ __forceinline__ double single_element_of_lane(const Onv<L> &x, const Onv<L> &y, int src, const double *__restrict__ h1e,
+                                                         const double *__restrict__ h2e, const ExcGeom &g, OrbLists &lists, bool &have_lists) {
+  if (!have_lists) {
+    build_lists<L>(x, g.sorb, g.noA, g.noB, lists, threadIdx.x & 31);
+    __syncwarp();
+    have_lists = true;
+  }
+  Onv<L> ys;
+#pragma unroll
+  for (int w = 0; w < L; ++w) ys.w[w] = __shfl_sync(0xffffffffu, y.w[w], src);
+  return single_element_warp<L, double>(x, ys, h1e, h2e, g.sorb, lists.occ_order, lists.n_occ);
+}
+
+// inclusive prefix sum of v over the lanes of the warp
+__device__ __forceinline__ u32 warp_inclusive_sum(u32 v) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const u32 up = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v += up;
+  }
+  return v;
+}
+
+// lanes hold consecutive segments of a list, incl = warp_inclusive_sum of their lengths: the lane whose segment holds entry e
+// (the first one whose inclusive prefix exceeds e; 31 when e is past the end)
+__device__ __forceinline__ int warp_segment_of(u32 incl, u32 e) {
+  int r = 0;
+#pragma unroll
+  for (int step = 16; step > 0; step >>= 1) {
+    const u32 v = __shfl_sync(0xffffffffu, incl, r + step - 1);
+    if (v <= e) r += step;
+  }
+  return r;
 }
 
 // alpha / beta strings of a one-word ONV from their 32-bit folds (inverse of fold_alpha / fold_beta)

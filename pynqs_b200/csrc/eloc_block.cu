@@ -404,12 +404,7 @@ eloc_block_kernel(const u64 *__restrict__ bra, const u32 *__restrict__ slots, co
           const int q = q0 + lane;
           u32 nb = 0;
           if (q >= q_part_lo && q < q_part_hi) nb = group_chunks(S.rng[q]);  // (the other parts' groups count as empty)
-          u32 incl = nb;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            const u32 up = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += up;
-          }
+          const u32 incl = warp_inclusive_sum(nb);
           if (q < sB) S.goff[q] = running + incl - nb;
           running += __shfl_sync(0xffffffffu, incl, 31);
         }

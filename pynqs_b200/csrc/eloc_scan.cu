@@ -342,14 +342,6 @@ eloc_scan_kernel(const u64 *__restrict__ bra, long long n, GroupView gv, HitRun 
     const u32 nc = (r.y - r.x + 31u) >> 5;
     return nc > sm.list_chunks ? (1u << 16) : nc;
   };
-  auto warp_scan = [&](u32 v) -> u32 {
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const u32 up = __shfl_up_sync(0xffffffffu, v, o);
-      if (lane >= o) v += up;
-    }
-    return v;
-  };
   // one round of groups (and not an empty slice): every thread keeps the work scan of its only group
   const bool one_round = q_hi > q_lo && q_hi - q_lo <= kScanThreads;
   u32 my_work = 0, my_incl = 0;
@@ -400,7 +392,7 @@ eloc_scan_kernel(const u64 *__restrict__ bra, long long n, GroupView gv, HitRun 
       }
     }
     my_work = work_of(q, r);
-    my_incl = warp_scan(my_work);
+    my_incl = warp_inclusive_sum(my_work);
     my_r = r;
     const u32 tot = __shfl_sync(0xffffffffu, my_incl, 31);
     if (lane == 0) wtot[(q0 - q_lo) / kScanThreads * kScanWarps + warp] = tot;
@@ -446,7 +438,7 @@ eloc_scan_kernel(const u64 *__restrict__ bra, long long n, GroupView gv, HitRun 
     __syncthreads();
     for (int q0 = q_lo; q0 < q_hi; q0 += kScanThreads) {  // the work counts again
       const int q = q0 + (int)threadIdx.x;
-      const u32 tot = __shfl_sync(0xffffffffu, warp_scan(work_of(q, q < q_hi ? rng[q] : make_uint2(0u, 0u))), 31);
+      const u32 tot = __shfl_sync(0xffffffffu, warp_inclusive_sum(work_of(q, q < q_hi ? rng[q] : make_uint2(0u, 0u))), 31);
       if (lane == 0) wtot[(q0 - q_lo) / kScanThreads * kScanWarps + warp] = tot;
     }
     __syncthreads();
@@ -499,7 +491,7 @@ eloc_scan_kernel(const u64 *__restrict__ bra, long long n, GroupView gv, HitRun 
       const int q = q0 + (int)threadIdx.x;
       const uint2 r = q < q_hi ? rng[q] : make_uint2(0u, 0u);
       const u32 mine = work_of(q, r);
-      place(q, r, mine, before + warp_scan(mine) - mine);
+      place(q, r, mine, before + warp_inclusive_sum(mine) - mine);
       for (int w = warp; w < kScanWarps; ++w) before += wtot[slot + w];
       slot += kScanWarps;
     }
@@ -684,64 +676,24 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
     for (int r0 = 0; r0 < nruns; r0 += 32) {
       HitRun mine = {0u, 0u};
       if (r0 + lane < nruns) mine = my_runs[r0 + lane];
-      u32 incl = mine.cnt;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const u32 up = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += up;
-      }
+      const u32 incl = warp_inclusive_sum(mine.cnt);
       const u32 total = __shfl_sync(0xffffffffu, incl, 31);
       for (u32 e0 = 0; e0 < total; e0 += 32) {
         const u32 e = e0 + (u32)lane;
-        int r = 0;  // the run that holds hit e: the first one whose inclusive prefix exceeds e
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1) {
-          const u32 v = __shfl_sync(0xffffffffu, incl, r + step - 1);
-          if (v <= e) r += step;
-        }
-        r = min(r, 31);
+        const int r = warp_segment_of(incl, e);  // the run that holds hit e
         const u32 r_incl = __shfl_sync(0xffffffffu, incl, r), r_cnt = __shfl_sync(0xffffffffu, mine.cnt, r);
         const u32 r_off = __shfl_sync(0xffffffffu, mine.off, r);
-        // (no early exits: the ballot below needs every lane)
+        // (no early exits: the ballot of the singles needs every lane)
         Onv<L> y = x;
-        long long id = 0;
+        u32 row = 0;
         int kind = 0;  // 1 single, 2 double, 0 nothing to add
-        if (e < total) {
-          const u32 h = hits[r_off + (e - (r_incl - r_cnt))];
-          const bool grouping = (h & kHitA) != 0u;
-          const u32 pos = HALF ? (h & kHitPos) : (h & ~kHitA);
-          y = load_onv<L>((grouping ? gv.keys[1] : gv.keys[0]) + (size_t)pos * L);
-          bool ok = true;
-          if (HALF) {  // the scan tested one folded string only: class of the full key vs the scan it came from
-            // (bitwise logic, no short-circuit branches: the lanes must stay together)
-            const u64 d = y.w[0] ^ x.w[0];
-            const int na = __popcll(d & kEven), nb = __popcll(d & kOdd);
-            const int moved = grouping ? nb : na, fixed = grouping ? na : nb;     // own-string scans: one string is x's
-            const bool ok_own = (fixed == 0) & ((moved == 2) | (moved == 4));     // single / same-spin double
-            const bool ok_ab = (na == 2) & (nb == 2);                             // alpha-beta double (bucket of a beta single)
-            ok = (h & kHitOwn) ? ok_own : ok_ab;
-          }
-          if (ok) {
-            kind = excitation_class<L>(x, y);
-            id = (long long)__ldg((grouping ? gv.rows[1] : gv.rows[0]) + pos);
-          }
-        }
-        if (kind == 2) accumulate<CPLX>(acc, load_psi<CPLX>(psi, id), p0, double_element<L, double>(x, y, h2e));
-        // single excitations (rare): one at a time by the whole warp, terms gathered in parallel
-        u32 pend = __ballot_sync(0xffffffffu, kind == 1);
-        while (pend) {
+        if (e < total) kind = decode_hit<L, HALF>(gv, x, hits[r_off + (e - (r_incl - r_cnt))], y, row);
+        if (kind == 2) accumulate<CPLX>(acc, load_psi<CPLX>(psi, row), p0, double_element<L, double>(x, y, h2e));
+        // single excitations: one at a time by the whole warp
+        for (u32 pend = __ballot_sync(0xffffffffu, kind == 1); pend; pend &= pend - 1u) {
           const int src = __ffs(pend) - 1;
-          pend &= pend - 1u;
-          if (!have_lists) {
-            build_lists<L>(x, g.sorb, g.noA, g.noB, s_lists[warp], lane);
-            __syncwarp();
-            have_lists = true;
-          }
-          Onv<L> ys;
-#pragma unroll
-          for (int w = 0; w < L; ++w) ys.w[w] = __shfl_sync(0xffffffffu, y.w[w], src);
-          const double v = single_element_warp<L, double>(x, ys, h1e, h2e, g.sorb, s_lists[warp].occ_order, s_lists[warp].n_occ);
-          if (lane == src) accumulate<CPLX>(acc, load_psi<CPLX>(psi, id), p0, v);
+          const double hs = single_element_of_lane<L>(x, y, src, h1e, h2e, g, s_lists[warp], have_lists);
+          if (lane == src) accumulate<CPLX>(acc, load_psi<CPLX>(psi, row), p0, hs);
         }
       }
     }
@@ -774,10 +726,10 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
 // empty ones.  The products (psi'/psi0) * H of a pass are summed per sample with a segmented shuffle scan (the hits of a
 // sample are adjacent) and the segment tails add into the sample's accumulator in shared memory -- a fixed order, no atomics.
 // Runs: round r of the outer loop takes run r of every sample of the tile (one or two rounds after the block kernel).
-// Samples flagged for the reference's route (overflow, duplicate keys) are then handled one by one by the whole warp.
 // Samples with long hit lists (a skewed table: thousands of hits for the samples of a heavy string, which sit next to each
 // other) would make one warp the tail of the launch: they are put on a list instead and the warp-per-sample kernel above
-// takes them, one warp each.
+// takes them, one warp each.  Samples flagged for the reference's route (overflow, duplicate keys) go on that list too, and
+// the kernel above takes the reference's route for them.
 constexpr u32 kHeavyHits = 256;
 
 struct EvalTileSmem {
@@ -789,7 +741,7 @@ struct EvalTileSmem {
 template <int L, bool CPLX, bool HALF>
 __global__ void __launch_bounds__(kEvalThreads)
 eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__restrict__ h1e, const double *__restrict__ h2e,
-                      const u64 *__restrict__ key, const double *__restrict__ psi, long long N, GroupView gv,
+                      const double *__restrict__ psi, GroupView gv,
                       const HitRun *__restrict__ runs, const u32 *__restrict__ run_cnt, int run_stride, const u32 *__restrict__ hits,
                       const u32 *__restrict__ self_pos, const double *__restrict__ hii, double *__restrict__ eloc,
                       double *__restrict__ psi0_out, u32 *__restrict__ heavy_list, ElocCounters *ctr, ExcGeom g, int per_warp) {
@@ -818,10 +770,9 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
   }
   // (the samples flagged for the reference's route go the same way: ~M binary searches each)
   const bool heavy = valid && (redo || my_hits > kHeavyHits);
-  redo = false;
   if (heavy) heavy_list[atomicAdd(&ctr->n_heavy, 1u)] = (u32)s;
   Cplx p0 = {0.0, 0.0};
-  if (valid && !redo && !heavy) {
+  if (valid && !heavy) {
     const u32 sp = self_pos[s];
     if (sp != kNoSelf) p0 = load_psi<CPLX>(psi, (long long)__ldg(gv.rows[0] + sp));
   }
@@ -831,62 +782,33 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
   T.p0[lane][1] = p0.im;
   {
     Cplx a0 = {0.0, 0.0};
-    if (valid && !redo && !heavy) accumulate<CPLX>(a0, p0, p0, hii[s]);  // row 0: (psi0 / psi0) * H_xx
+    if (valid && !heavy) accumulate<CPLX>(a0, p0, p0, hii[s]);  // row 0: (psi0 / psi0) * H_xx
     T.acc[lane][0] = a0.re;
     T.acc[lane][1] = a0.im;
   }
   __syncwarp();
-  const int max_runs = __reduce_max_sync(0xffffffffu, (redo || heavy) ? 0 : nruns);
+  const int max_runs = __reduce_max_sync(0xffffffffu, heavy ? 0 : nruns);
   int lists_owner = -1;
   for (int r = 0; r < max_runs; ++r) {
     HitRun mine = {0u, 0u};
-    if (!redo && !heavy && r < nruns) mine = my_runs[r];
-    u32 incl = mine.cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const u32 up = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += up;
-    }
+    if (!heavy && r < nruns) mine = my_runs[r];
+    const u32 incl = warp_inclusive_sum(mine.cnt);
     const u32 total = __shfl_sync(0xffffffffu, incl, 31);
     for (u32 e0 = 0; e0 < total; e0 += 32) {
       const u32 e = e0 + (u32)lane;
-      int j = 0;  // the sample that holds hit e: the first one whose inclusive prefix exceeds e
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const u32 v = __shfl_sync(0xffffffffu, incl, j + step - 1);
-        if (v <= e) j += step;
-      }
-      j = min(j, 31);
+      const int j = warp_segment_of(incl, e);  // the sample that holds hit e
       const u32 j_incl = __shfl_sync(0xffffffffu, incl, j), j_cnt = __shfl_sync(0xffffffffu, mine.cnt, j);
       const u32 j_off = __shfl_sync(0xffffffffu, mine.off, j);
       Onv<L> xs, y;
 #pragma unroll
       for (int w = 0; w < L; ++w) xs.w[w] = T.x[j][w];
       y = xs;
-      long long id = 0;
+      u32 row = 0;
       int kind = 0;  // 1 single, 2 double, 0 nothing to add
-      if (e < total) {
-        const u32 h = hits[j_off + (e - (j_incl - j_cnt))];
-        const bool grouping = (h & kHitA) != 0u;
-        const u32 pos = HALF ? (h & kHitPos) : (h & ~kHitA);
-        y = load_onv<L>((grouping ? gv.keys[1] : gv.keys[0]) + (size_t)pos * L);
-        bool ok = true;
-        if (HALF) {  // the scan tested one folded string only: class of the full key vs the scan it came from
-          const u64 d = y.w[0] ^ xs.w[0];
-          const int na = __popcll(d & kEven), nb = __popcll(d & kOdd);
-          const int moved = grouping ? nb : na, fixed = grouping ? na : nb;
-          const bool ok_own = (fixed == 0) & ((moved == 2) | (moved == 4));
-          const bool ok_ab = (na == 2) & (nb == 2);
-          ok = (h & kHitOwn) ? ok_own : ok_ab;
-        }
-        if (ok) {
-          kind = excitation_class<L>(xs, y);
-          id = (long long)__ldg((grouping ? gv.rows[1] : gv.rows[0]) + pos);
-        }
-      }
+      if (e < total) kind = decode_hit<L, HALF>(gv, xs, hits[j_off + (e - (j_incl - j_cnt))], y, row);
       Cplx v = {0.0, 0.0};
       const Cplx pj = {T.p0[j][0], T.p0[j][1]};
-      if (kind == 2) accumulate<CPLX>(v, load_psi<CPLX>(psi, id), pj, double_element<L, double>(xs, y, h2e));
+      if (kind == 2) accumulate<CPLX>(v, load_psi<CPLX>(psi, row), pj, double_element<L, double>(xs, y, h2e));
       // single excitations (rare): one at a time by the whole warp, terms gathered in parallel
       u32 pend = __ballot_sync(0xffffffffu, kind == 1);
       while (pend) {
@@ -906,7 +828,7 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
           lists_owner = js;
         }
         const double hv = single_element_warp<L, double>(xb, yb, h1e, h2e, g.sorb, s_lists[warp].occ_order, s_lists[warp].n_occ);
-        if (lane == src) accumulate<CPLX>(v, load_psi<CPLX>(psi, id), pj, hv);
+        if (lane == src) accumulate<CPLX>(v, load_psi<CPLX>(psi, row), pj, hv);
       }
       // sum of v over the lanes of the same sample (adjacent), then the last lane of every sample adds it in
       const int jkey = e < total ? j : 32 + lane;  // idle lanes: segments of their own
@@ -929,39 +851,7 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
     }
   }
   __syncwarp();
-  Cplx acc = {T.acc[lane][0], T.acc[lane][1]};
-  // ---- the reference's route for flagged samples: every excitation in row order, classic binary search ----------------------
-  u32 todo = __ballot_sync(0xffffffffu, valid && redo);
-  while (todo) {
-    const int src = __ffs(todo) - 1;
-    todo &= todo - 1u;
-    Onv<L> xb;
-#pragma unroll
-    for (int w = 0; w < L; ++w) xb.w[w] = T.x[src][w];
-    __syncwarp();
-    build_lists<L>(xb, g.sorb, g.noA, g.noB, s_lists[warp], lane);
-    __syncwarp();
-    lists_owner = src;
-    const OrbLists &lists = s_lists[warp];
-    Cplx q0 = {0.0, 0.0}, a = {0.0, 0.0};
-    const long long id0 = classic_search<L>(key, N, xb);
-    if (id0 >= 0) q0 = load_psi<CPLX>(psi, id0);
-    if (lane == 0) accumulate<CPLX>(a, q0, q0, hii[s0 + src]);
-    for (int r = lane; r < g.nsd; r += 32) {
-      const Exc ex = decode_exc(g, lists, r);
-      const long long id = classic_search<L>(key, N, apply_exc<L>(xb, ex));
-      if (id >= 0) accumulate<CPLX>(a, load_psi<CPLX>(psi, id), q0, exc_element<L, double>(xb, ex, h1e, h2e, g.sorb));
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      a.re += __shfl_xor_sync(0xffffffffu, a.re, o);
-      if (CPLX) a.im += __shfl_xor_sync(0xffffffffu, a.im, o);
-    }
-    if (lane == src) {
-      acc = a;
-      p0 = q0;
-    }
-  }
+  const Cplx acc = {T.acc[lane][0], T.acc[lane][1]};
   if (valid && !heavy) {
     if (CPLX) {
       eloc[2 * s] = acc.re;
@@ -1132,7 +1022,7 @@ static int launch_eloc_LC(const u64 *bra, long long n, const double *h1e, const 
       const int per_warp = 32;
       const long long per_cta = (long long)per_warp * (kEvalThreads / 32);
       const unsigned eb = (unsigned)((nb + per_cta - 1) / per_cta);
-      eloc_eval_tile_kernel<L, CPLX, HALF><<<eb, kEvalThreads, 0, st>>>(bra + b0 * L, nb, h1e, h2e, key, psi, N, gv, runs, run_cnt,
+      eloc_eval_tile_kernel<L, CPLX, HALF><<<eb, kEvalThreads, 0, st>>>(bra + b0 * L, nb, h1e, h2e, psi, gv, runs, run_cnt,
                                                                         lay.run_stride, hits, self_pos, hii + b0, eloc + b0 * w,
                                                                         psi0 + b0 * w, heavy, ctr, g, per_warp);
       count_launch();

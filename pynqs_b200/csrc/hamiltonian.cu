@@ -96,21 +96,11 @@ hamiltonian_row_kernel(const u64 *__restrict__ bra, long long n, const double *_
         double v = 0.0;
         if (EMIT) {
           if (kind == 2) v = double_element<L, double>(x, y, h2e);
-          // single excitations (rare): one at a time by the whole warp, terms gathered in parallel
-          u32 pend = __ballot_sync(0xffffffffu, kind == 1);
-          while (pend) {
+          // single excitations: one at a time by the whole warp
+          for (u32 pend = __ballot_sync(0xffffffffu, kind == 1); pend; pend &= pend - 1u) {
             const int src = __ffs(pend) - 1;
-            pend &= pend - 1u;
-            if (!have_lists) {
-              build_lists<L>(x, g.sorb, g.noA, g.noB, lists, lane);
-              __syncwarp();
-              have_lists = true;
-            }
-            Onv<L> ys;
-#pragma unroll
-            for (int w = 0; w < L; ++w) ys.w[w] = __shfl_sync(0xffffffffu, y.w[w], src);
-            const double hv = single_element_warp<L, double>(x, ys, h1e, h2e, g.sorb, lists.occ_order, lists.n_occ);
-            if (lane == src) v = hv;
+            const double hs = single_element_of_lane<L>(x, y, src, h1e, h2e, g, lists, have_lists);
+            if (lane == src) v = hs;
           }
         }
         put(kind != 0, (long long)row, v);
