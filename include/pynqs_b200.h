@@ -193,6 +193,27 @@ int pynqs_csr_spmm(const int64_t *crow, const int64_t *col, const double *val, i
 int pynqs_spin_square_apply(const uint8_t *bra, int64_t n, int sorb, const uint8_t *key, int64_t N, const void *group_ws,
                             const double *X, int64_t ldx, int k, double *Y, int64_t ldy, void *stream);
 
+/* Additive op: the off-diagonal part of the one- and two-body reduced density matrices of c over the sorted key table
+ * (N keys of (sorb - 1) / 64 + 1 words), summed over the entries (i, j != i) of a square CSR structure crow int64 [N + 1],
+ * col int64 [nnz] -- the structure of pynqs_hamiltonian_emit with bra = key, whose entries are exactly the table pairs
+ * connected by a single or double excitation.  c: N values, double (c_complex = 0) or interleaved (re, im) doubles
+ * (c_complex = 1).  Orbital p has alpha at bit 2p and beta at bit 2p + 1, norb = sorb / 2; the sign counts the occupied
+ * bits below each operator's bit.  Not normalised, and without the diagonal i == j, which the caller adds (|c_i|^2 times
+ * occupation products).  Outputs, in c's element type, row-major, overwritten (zero where no off-diagonal pair lands):
+ *   dm1 [2][norb][norb]            dm1[s][p][q] = sum conj(c_i) c_j <key_i| a+_{q s} a_{p s} |key_j>, s = alpha, beta;
+ *   dm2 [3][norb][norb][norb][norb] (aa, ab, bb), or NULL for dm1 alone:
+ *                                  dm2[st][p][q][r][s] = sum conj(c_i) c_j <key_i| a+_{p s} a+_{r t} a_{s t} a_{q s} |key_j>
+ * (PySCF's make_rdm12s layout).  Entries that are not a single or double excitation, or change the spin, add nothing.
+ * Deterministic (identical bits on every call, no float atomics): one record per CSR entry, a stable radix sort by output
+ * bin, one warp per bin summing in the bin's order.  No host synchronisation.  scratch: pynqs_rdm_scratch_bytes(N, nnz,
+ * sorb) = 24 nnz + 4 nnz (records, double-buffered, and run starts) + 2 nnz + 4 MiB (sort / run-length / scan
+ * temporaries) + alignment; it does not depend on c's type or on dm2.  PYNQS_EVALUE, before anything touches the device,
+ * for an odd sorb or one outside (0, PYNQS_MAX_SORB], N or nnz < 0 or >= 2^31, c_complex not 0 / 1, a NULL bytes / dm1,
+ * crow / key / c (N > 0) or col / scratch (nnz > 0).  A table with duplicate keys is the caller's to refuse. */
+int pynqs_rdm_scratch_bytes(int64_t N, int64_t nnz, int sorb, int64_t *bytes);
+int pynqs_rdm_offdiag(const int64_t *crow, const int64_t *col, const uint8_t *key, int64_t N, int64_t nnz, int sorb, const double *c,
+                      int c_complex, void *scratch, int64_t scratch_bytes, double *dm1, double *dm2, void *stream);
+
 /* ---- REDUCE method (vmc/energy/eloc.py:257-297, additive) -----------------------------------------
  * The reference materialises comb [n, M, 8L] and Hmat [n, M] and keeps torch.where(|Hmat| >= eps).  These
  * entry points return the kept rows only, in the same (ascending flat index s * M + m) order:

@@ -761,6 +761,40 @@ def spin_square_matmul(bra: Tensor, sorb: int, bra_key: Tensor, X: Tensor, group
     return _from_real_block(Y, X)
 
 
+def rdm_offdiag(crow: Tensor, col: Tensor, bra_key: Tensor, c: Tensor, sorb: int, two_body: bool = True) -> Tuple[Tensor, "Tensor | None"]:
+    """The off-diagonal part of the reduced density matrices of c over the sorted table (pynqs_rdm_offdiag): the sums over
+    the entries (i, j != i) of the square CSR structure crow int64 [N + 1] / col int64 [nnz] (sample_space_hamiltonian with
+    bra = bra_key) of conj(c_i) c_j <key_i| ... |key_j>, not normalised.  Returns dm1 [2, norb, norb] (alpha, beta) and dm2
+    [3, norb, norb, norb, norb] (aa, ab, bb) in PySCF's make_rdm12s layout, or None when not two_body; c's dtype (float64 or
+    complex128).  Deterministic (identical bits on every call); one host synchronisation (nnz)."""
+    dev = _need_cuda(crow, col, bra_key, c)
+    if crow.dtype != torch.int64 or col.dtype != torch.int64:
+        raise ValueError("crow and col must be int64")
+    if bra_key.dim() != 2 or crow.dim() != 1 or crow.numel() != bra_key.size(0) + 1 or col.dim() != 1:
+        raise ValueError("bra_key must be 2-D [N, 8L], crow 1-D [N + 1], col 1-D")
+    if c.dtype not in (torch.float64, torch.complex128) or c.shape != (bra_key.size(0),):
+        raise ValueError(f"c must be float64 or complex128 [N] with N = {bra_key.size(0)}")
+    for t, nm in ((crow, "crow"), (col, "col"), (bra_key, "bra_key"), (c, "c")):
+        _contig(t, nm)
+    _check_width(bra_key, sorb, "bra_key")
+    N, norb = bra_key.size(0), sorb // 2
+    nnz = int(crow[N].item())
+    if nnz != col.numel():
+        raise ValueError(f"crow[N] = {nnz} does not match col's {col.numel()} entries")
+    cr = torch.view_as_real(c.resolve_conj()) if c.is_complex() else c
+    dm1 = torch.empty((2, norb, norb), dtype=c.dtype, device=dev)
+    dm2 = torch.empty((3, norb, norb, norb, norb), dtype=c.dtype, device=dev) if two_body else None
+    lib = _lib.load()
+    nbytes = _lib.ctypes.c_int64()
+    _lib.check(lib.pynqs_rdm_scratch_bytes(i64(N), i64(nnz), int(sorb), _lib.ctypes.byref(nbytes)))
+    scratch = torch.empty(nbytes.value, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.pynqs_rdm_offdiag(vp(crow.data_ptr()), vp(col.data_ptr()), vp(bra_key.data_ptr()), i64(N), i64(nnz), int(sorb),
+                                         vp(cr.data_ptr()), int(c.is_complex()), vp(scratch.data_ptr()), i64(nbytes.value),
+                                         vp(dm1.data_ptr()), vp(dm2.data_ptr() if two_body else None), _stream(dev)))
+    return dm1, dm2
+
+
 def lookup_compact(idx_array: Tensor, mask: Tensor, wf_value: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
     """(positions with mask set, positions without, wf_value[idx_array[mask]]) -- the index glue of
     WavefunctionLUT.lookup (utils/public_function.py:825-838: arange, two boolean-mask selections, masked_select, gather)

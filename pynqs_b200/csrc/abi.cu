@@ -85,6 +85,9 @@ int launch_csr_spmm(const long long *, const long long *, const double *, long l
                     cudaStream_t);
 int launch_spin_square(const u64 *, long long, int, const u64 *, long long, const void *, const double *, long long, int, double *,
                        long long, cudaStream_t);
+long long rdm_scratch_bytes(long long);
+int launch_rdm(const long long *, const long long *, const u64 *, long long, long long, int, const double *, int, void *, long long, double *,
+               double *, cudaStream_t);
 
 static int check_geometry(int sorb, int nele, int noA, int noB) {
   if (sorb <= 0 || sorb > PYNQS_MAX_SORB) {
@@ -481,6 +484,50 @@ int pynqs_spin_square_apply(const uint8_t *bra, int64_t n, int sorb, const uint8
   }
   return launch_spin_square(reinterpret_cast<const u64 *>(bra), n, (sorb - 1) / 64 + 1, reinterpret_cast<const u64 *>(key), N, group_ws, X,
                             ldx, k, Y, ldy, (cudaStream_t)stream);
+}
+
+static int rdm_check(const char *what, int64_t N, int64_t nnz, int sorb) {
+  if (sorb <= 0 || sorb > PYNQS_MAX_SORB || (sorb & 1)) {
+    set_error("%s: sorb = %d must be even and in (0, %d]", what, sorb, PYNQS_MAX_SORB);
+    return PYNQS_EVALUE;
+  }
+  if (N < 0 || N >= (1LL << 31) || nnz < 0 || nnz >= (1LL << 31)) {
+    set_error("%s: bad N = %lld or nnz = %lld (both < 2^31)", what, (long long)N, (long long)nnz);
+    return PYNQS_EVALUE;
+  }
+  return 0;
+}
+
+int pynqs_rdm_scratch_bytes(int64_t N, int64_t nnz, int sorb, int64_t *bytes) {
+  if (int rc = rdm_check("rdm_scratch_bytes", N, nnz, sorb)) return rc;
+  if (bytes == nullptr) {
+    set_error("rdm_scratch_bytes: null bytes");
+    return PYNQS_EVALUE;
+  }
+  *bytes = rdm_scratch_bytes(nnz);
+  return 0;
+}
+
+int pynqs_rdm_offdiag(const int64_t *crow, const int64_t *col, const uint8_t *key, int64_t N, int64_t nnz, int sorb, const double *c,
+                      int c_complex, void *scratch, int64_t scratch_bytes, double *dm1, double *dm2, void *stream) {
+  if (int rc = rdm_check("rdm_offdiag", N, nnz, sorb)) return rc;
+  if (c_complex != 0 && c_complex != 1) {
+    set_error("rdm_offdiag: c_complex = %d must be 0 or 1", c_complex);
+    return PYNQS_EVALUE;
+  }
+  if (dm1 == nullptr || (N > 0 && (crow == nullptr || key == nullptr || c == nullptr)) ||
+      (nnz > 0 && (col == nullptr || scratch == nullptr))) {
+    set_error("rdm_offdiag: null pointer (dm1; crow / key / c for N > 0; col / scratch for nnz > 0)");
+    return PYNQS_EVALUE;
+  }
+  const size_t norb = (size_t)(sorb / 2), el = c_complex ? 16 : 8;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (cudaMemsetAsync(dm1, 0, 2 * norb * norb * el, st) != cudaSuccess ||
+      (dm2 != nullptr && cudaMemsetAsync(dm2, 0, 3 * norb * norb * norb * norb * el, st) != cudaSuccess))
+    return check_launch("rdm_offdiag: memset of dm1 / dm2");
+  if (N == 0 || nnz == 0) return 0;
+  return launch_rdm(reinterpret_cast<const long long *>(crow), reinterpret_cast<const long long *>(col), reinterpret_cast<const u64 *>(key), N,
+                    nnz, sorb, c, c_complex, scratch, scratch_bytes, dm1, dm2, st);
 }
 
 int64_t pynqs_reduce_scratch_bytes(int64_t n) { return reduce_scratch_bytes(n); }

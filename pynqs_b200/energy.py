@@ -160,6 +160,67 @@ def spin_square(WF_LUT: WavefunctionLUT, C: Tensor, sorb: int) -> Tensor:
     return (C.conj() * S2C).sum(0).real / (C.conj() * C).sum(0).real
 
 
+def make_rdm1s(WF_LUT: WavefunctionLUT, C: Tensor, sorb: int, H: Tensor) -> Tuple[Tensor, Tensor]:
+    """The one-body reduced density matrices (dm1a, dm1b) of the state C over the table, dm1s[p, q] = <c|a+_qs a_ps|c> / <c|c>
+    (PySCF's make_rdm1s): see make_rdm12s for the arguments and conventions.  Skips the two-body work; its dm1 has the bits
+    of make_rdm12s's.  The natural occupations are eigvalsh(dm1a + dm1b)."""
+    dm1, _ = _make_rdm(WF_LUT, C, sorb, H, False)
+    return dm1[0], dm1[1]
+
+
+def make_rdm12s(WF_LUT: WavefunctionLUT, C: Tensor, sorb: int, H: Tensor) -> Tuple[Tuple[Tensor, Tensor], Tuple[Tensor, Tensor, Tensor]]:
+    """The one- and two-body reduced density matrices of the state C over the table, in PySCF's make_rdm12s conventions:
+    ((dm1a, dm1b), (dm2aa, dm2ab, dm2bb)) with dm1s[p, q] = <c|a+_qs a_ps|c> / <c|c> ([norb, norb], norb = sorb / 2) and
+    dm2st[p, q, r, s] = <c|a+_ps a+_rt a_st a_qs|c> / <c|c> ([norb]^4).  Orbital p has alpha at bit 2p and beta at 2p + 1,
+    and the sign is get_hij_torch's.  Sums run over pairs of table rows only -- the sample-space convention of
+    local_energy_sample_space and spin_square: a determinant outside the table counts as c = 0 --, so with H the energy
+    sum h (dm1a + dm1b) + 1/2 sum eri dm2aa + sum eri dm2ab + 1/2 sum eri dm2bb equals Re(c^H H c) / c^H c.  The natural
+    occupations are eigvalsh(dm1a + dm1b).
+
+    C: float64 or complex128 [N], rows in the order of WF_LUT.bra_key (a CI root of sample_space_ground_state, or
+    WF_LUT.wf_value); the result has C's dtype (complex dm1 is Hermitian).  H: the square
+    sample_space_hamiltonian(WF_LUT.bra_key, ...) of the same table, of which only the structure is read.  ValueError when
+    H is not (N, N) CSR, C has the wrong shape or dtype, sum |c|^2 = 0, or the table has duplicate keys.  Deterministic
+    (identical bits on every call); two host synchronisations."""
+    dm1, dm2 = _make_rdm(WF_LUT, C, sorb, H, True)
+    return (dm1[0], dm1[1]), (dm2[0], dm2[1], dm2[2])
+
+
+def _make_rdm(WF_LUT: WavefunctionLUT, C: Tensor, sorb: int, H: Tensor, two_body: bool) -> Tuple[Tensor, "Tensor | None"]:
+    keys = WF_LUT.bra_key
+    N = keys.size(0)
+    if H.layout != torch.sparse_csr or tuple(H.shape) != (N, N):
+        raise ValueError(f"H must be a sparse CSR tensor of shape ({N}, {N})")
+    if C.dtype not in (torch.float64, torch.complex128) or C.shape != (N,):
+        raise ValueError(f"C must be float64 or complex128 of shape ({N},), got {C.dtype} {tuple(C.shape)}")
+    w = torch.view_as_real(C).square().sum(1) if C.is_complex() else C * C  # |c_i|^2
+    norm = w.sum()
+    dup = (keys[1:] == keys[:-1]).all(1).any() if N > 1 else torch.zeros((), dtype=torch.bool, device=keys.device)
+    zero, has_dup = torch.stack([norm == 0, dup]).tolist()
+    if zero:
+        raise ValueError("C has sum |c|^2 = 0")
+    if has_dup:
+        raise ValueError("the table has duplicate keys")
+    dm1, dm2 = ops.rdm_offdiag(H.crow_indices(), H.col_indices(), keys, C.contiguous(), sorb, two_body)
+    # the diagonal pairs: |c_i|^2 times occupation products, as dense products over the occupations Occ [N, 2, norb]
+    norb = sorb // 2
+    bits = (keys.unsqueeze(2) >> torch.arange(8, device=keys.device, dtype=torch.uint8)) & 1
+    occ = bits.view(N, -1)[:, :sorb].view(N, norb, 2).permute(0, 2, 1).contiguous().to(torch.float64)
+    ar = torch.arange(norb, device=keys.device)
+    dm1[:, ar, ar] += (w @ occ.view(N, 2 * norb)).view(2, norb).to(dm1.dtype)
+    if two_body:
+        wocc = occ * w.view(N, 1, 1)
+        for blk, (s, t) in enumerate(((0, 0), (0, 1), (1, 1))):
+            G = (wocc[:, s].T @ occ[:, t]).to(dm2.dtype)  # sum |c_i|^2 n_ps n_rt
+            if s == t:
+                G.fill_diagonal_(0)  # a+_p a+_p = 0
+                dm2[blk, ar[:, None], ar[None, :], ar[None, :], ar[:, None]] -= G  # <a+_p a+_r a_p a_r> = -n_p n_r
+            dm2[blk, ar[:, None], ar[:, None], ar[None, :], ar[None, :]] += G
+        dm2 /= norm
+    dm1 /= norm
+    return dm1, dm2
+
+
 def local_energy_three_call(x: Tensor, h1e: Tensor, h2e: Tensor, WF_LUT: WavefunctionLUT, sorb: int, nele: int,
                             noa: int, nob: int, dtype=torch.double, batch: int = 4096) -> Tuple[Tensor, Tensor, Tensor]:
     """The reference's op sequence (eloc.py:369-397) in chunks of `batch` samples."""
