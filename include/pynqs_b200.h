@@ -236,9 +236,11 @@ int pynqs_reduce_eloc(const void *psi, int psi_complex, const double *hij, const
 /* Stochastic / semi-stochastic branch of the REDUCE method (vmc/energy/eloc.py:257-283, eps_sample > 0; what every
  * shipped input selects, main.py:149-159): per sample, eps_sample draws from p(m) ~ |H_m| over the rows with |H_m| < eps
  * (all rows when eps == 0); a drawn row's element becomes (count / eps_sample) * H_m / p(m) = sign(H_m) * S * count /
- * eps_sample with S the sample's sum of sub-eps magnitudes; rows with |H_m| >= eps (eps > 0) are kept exactly.  Same
- * count / emit protocol and outputs as pynqs_reduce_count / _emit; per sample the kept rows come first (ascending m), then
- * the drawn rows (ascending m).  No [n, M] array and no [n, eps_sample] array is materialised.
+ * eps_sample with S the sample's sum of sub-eps magnitudes; rows with |H_m| >= eps (eps > 0) are kept exactly.  eps is
+ * compared in the integrals' dtype (as torch compares Hmat, and as pynqs_reduce_count does): under float32 the threshold
+ * is (float)eps.  A sample with S = 0 (every row kept or exactly zero) has nothing drawn; the generator never draws a row
+ * with H_m == 0.  Same count / emit protocol and outputs as pynqs_reduce_count / _emit; per sample the kept rows come
+ * first (ascending m), then the drawn rows (ascending m).  No [n, M] array and no [n, eps_sample] array is materialised.
  * Draws: Philox4x32-10 keyed by `seed` (reproducible; not torch.multinomial's stream), or -- draws != NULL -- the caller's
  * row indices int64[n, eps_sample] (what torch.multinomial returned), which makes the result a deterministic function of
  * the inputs.  eps_sample <= 8192.  scratch: pynqs_reduce_sample_scratch_bytes(n) bytes, the same buffer for both calls. */

@@ -320,7 +320,9 @@ def get_comb_hij_sampled(bra: Tensor, h1e: Tensor, h2e: Tensor, sorb: int, nele:
                          *, seed: int | None = None, draws: Tensor | None = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """Additive op for the stochastic / semi-stochastic REDUCE method (vmc/energy/eloc.py:257-283, eps_sample > 0):
     per sample, eps_sample draws from p(m) ~ |H_m| over the rows with |H_m| < eps (all rows if eps == 0); the element of a
-    drawn row becomes (count / eps_sample) * H_m / p(m); rows with |H_m| >= eps (eps > 0) are kept exactly.
+    drawn row becomes (count / eps_sample) * H_m / p(m); rows with |H_m| >= eps (eps > 0) are kept exactly.  eps is compared
+    in the integrals' dtype, like torch.where(|Hmat| >= eps) and get_comb_hij_reduced.  A sample whose sub-eps magnitudes
+    sum to 0 has nothing drawn (where torch.multinomial would raise); the generator never draws a row with H_m == 0.
     Returns (x uint8 [K, 8L], hij [K], gt_eps_idx int64 [K], offsets int64 [n + 1]) like get_comb_hij_reduced; per sample the
     kept rows (ascending) come first, then the drawn ones (ascending).  Nothing of size [n, M] or [n, eps_sample] is stored.
     seed: Philox key (default: drawn from torch's CPU generator, so torch.manual_seed makes runs reproducible);

@@ -1,6 +1,7 @@
 // reduce_sample.cu -- the stochastic / semi-stochastic branch of the REDUCE method (vmc/energy/eloc.py:257-283):
 //
-//   hij = |Hmat| with the entries >= eps zeroed (eps > 0: semi-stochastic; those entries are kept exactly)
+//   hij = |Hmat| with the entries >= eps zeroed (eps > 0: semi-stochastic; those entries are kept exactly; eps is rounded
+//         to the integrals' dtype first, as torch compares in the tensor's dtype)
 //   p[n, m] = hij / hij.sum(1);   eps_sample draws per sample from p (torch.multinomial, with replacement)
 //   Hmat[n, m] <- (count[n, m] / eps_sample) * Hmat[n, m] / p[n, m]     for the drawn (n, m)
 //   kept set = {|Hmat| >= eps}  U  {drawn}
@@ -102,6 +103,9 @@ reduce_sample_kernel(const u64 *__restrict__ bra, const T *__restrict__ h1e, con
   const int M = g.nsd + 1;
   const T hii = diag[s];
   const bool semi = eps > 0.0;  // eps == 0: purely stochastic, nothing is kept deterministically (eloc.py:263-270)
+  // |H| is compared with eps rounded to the integrals' dtype, as torch compares Hmat and as reduce_kernel does: under float32
+  // a row with |H| == float(eps) < eps is kept.  Both passes use this one value, so counts and emitted rows agree.
+  const double thr = (double)(T)eps;
 
   // running sum of the sub-eps magnitudes in row order: the same code (same rounding) in every pass
   auto chunk_scan = [&](double w, double &running, double &before) {
@@ -133,7 +137,7 @@ reduce_sample_kernel(const u64 *__restrict__ bra, const T *__restrict__ h1e, con
       if (m < M) {
         Onv<L> ket;
         const double a = fabs((double)row_value<L, T>(x, g, lists, h1e, h2e, hii, m, ket));
-        w = (semi && a >= eps) ? 0.0 : a;
+        w = (semi && a >= thr) ? 0.0 : a;
       }
       chunk_scan(w, running, before);
     }
@@ -190,7 +194,7 @@ reduce_sample_kernel(const u64 *__restrict__ bra, const T *__restrict__ h1e, con
     if (m < M) {
       v = row_value<L, T>(x, g, lists, h1e, h2e, hii, m, ket);
       const double a = fabs((double)v);
-      keep = semi && a >= eps;
+      keep = semi && a >= thr;
       w = keep ? 0.0 : a;
     }
     chunk_scan(w, running, before);
