@@ -88,9 +88,7 @@ __device__ __forceinline__ int decode_hit(const GroupView &gv, const Onv<L> &x, 
 
 // <x|H|y> of lane src's single excitation x -> y, evaluated by the whole warp (every lane passes the same x; every lane gets
 // the element).  The warp's orbital lists of x are built at the first single of the sample; have_lists remembers that.
-// The callers walk their singles (rare) with a ballot and use the element inside that loop.  (A helper that returned each
-// lane's element after the loop kept one more value live through it: ptxas for sm_100a then gave eloc_eval_kernel<1, false, *>
-// 60 / 64 bytes of spill stores / loads instead of 48 / 48 at its 40-register bound.)
+// The caller (hamiltonian_row_kernel) walks its singles (rare) with a ballot and uses the element inside that loop.
 template <int L>
 __device__ __forceinline__ double single_element_of_lane(const Onv<L> &x, const Onv<L> &y, int src, const double *__restrict__ h1e,
                                                          const double *__restrict__ h2e, const ExcGeom &g, OrbLists &lists, bool &have_lists) {

@@ -620,6 +620,37 @@ eloc_scan_kernel(const u64 *__restrict__ bra, long long n, GroupView gv, HitRun 
 }
 
 // ---- evaluation ---------------------------------------------------------------------------------------------
+// Single excitations are rare (under 2 % of the hits of the benchmarked Fe2S2 tables) but cost ~30 two-electron terms each.  The
+// passes over the hit list put them on a per-warp queue (ballot + popcount) and go on; when the next pass's singles would not fit,
+// and when the hit list ends, the queue is flushed: lane i evaluates entry i (single_element, one lane per single).
+template <int L>
+struct SingleQueue {
+  u64 y[32][L];  // the key
+  u32 row[32];   // its row of the sorted table
+  u32 j[32];     // 32-samples-per-warp kernel: the sample of the tile it belongs to
+};
+
+// the lanes with a single (kind == 1) append it to the queue; flush(qn) empties a queue of qn entries first when they would
+// not fit.  Every lane of the warp calls this.
+template <int L, typename Flush>
+__device__ __forceinline__ void push_singles(SingleQueue<L> &q, u32 &qn, int kind, const Onv<L> &y, u32 row, u32 j, Flush flush) {
+  const u32 m = __ballot_sync(0xffffffffu, kind == 1);
+  if (m == 0u) return;
+  if (qn + (u32)__popc(m) > 32u) {
+    flush(qn);
+    qn = 0;
+  }
+  if (kind == 1) {
+    const u32 at = qn + (u32)__popc(m & ((1u << (threadIdx.x & 31)) - 1u));
+#pragma unroll
+    for (int w = 0; w < L; ++w) q.y[at][w] = y.w[w];
+    q.row[at] = row;
+    q.j[at] = j;
+  }
+  qn += (u32)__popc(m);
+  __syncwarp();
+}
+
 // (launch bounds per variant: the 40-register budget that lets 12 CTAs of the real one-word kernel share an SM makes the
 //  complex and multi-word variants spill 250-390 bytes; they get 80 registers instead)
 template <int L, bool CPLX, bool HALF>
@@ -630,6 +661,7 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
                  const u32 *__restrict__ self_pos, const double *__restrict__ hii, double *__restrict__ eloc,
                  double *__restrict__ psi0_out, const u32 *__restrict__ list, ElocCounters *ctr, ExcGeom g) {
   __shared__ OrbLists s_lists[kEvalThreads / 32];
+  __shared__ SingleQueue<L> s_queue[kEvalThreads / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // work items: every sample of the call (one per warp), or (list != nullptr) the samples the tile kernel put on the list of
   // long hit lists, handed out one by one (their lengths differ by orders of magnitude)
@@ -667,10 +699,21 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
       if (id >= 0) accumulate<CPLX>(acc, load_psi<CPLX>(psi, id), p0, exc_element<L, double>(x, e, h1e, h2e, g.sorb));
     }
   } else {
-    bool have_lists = false;
     const u32 sp = self_pos[s];
     if (sp != kNoSelf) p0 = load_psi<CPLX>(psi, (long long)__ldg(gv.rows[0] + sp));
     if (lane == 0) accumulate<CPLX>(acc, p0, p0, hii[s]);  // row 0: (psi0/psi0) * H_xx
+    SingleQueue<L> &q = s_queue[warp];
+    u32 qn = 0;
+    // lane i: entry i, into its own accumulator (two terms in flight: more spill at the real one-word kernel's 40 registers)
+    auto flush = [&](u32 cnt) {
+      if ((u32)lane < cnt) {
+        Onv<L> yq;
+#pragma unroll
+        for (int w = 0; w < L; ++w) yq.w[w] = q.y[lane][w];
+        accumulate<CPLX>(acc, load_psi<CPLX>(psi, q.row[lane]), p0, single_element<L, 2, double>(x, yq, h1e, h2e, g.sorb));
+      }
+      __syncwarp();
+    };
     // the sample's runs back to back: lane r holds run r and an inclusive prefix of the counts, so the
     // whole list is walked 32 hits at a time whatever the runs' lengths (32 runs per round)
     for (int r0 = 0; r0 < nruns; r0 += 32) {
@@ -689,14 +732,10 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
         int kind = 0;  // 1 single, 2 double, 0 nothing to add
         if (e < total) kind = decode_hit<L, HALF>(gv, x, hits[r_off + (e - (r_incl - r_cnt))], y, row);
         if (kind == 2) accumulate<CPLX>(acc, load_psi<CPLX>(psi, row), p0, double_element<L, double>(x, y, h2e));
-        // single excitations: one at a time by the whole warp
-        for (u32 pend = __ballot_sync(0xffffffffu, kind == 1); pend; pend &= pend - 1u) {
-          const int src = __ffs(pend) - 1;
-          const double hs = single_element_of_lane<L>(x, y, src, h1e, h2e, g, s_lists[warp], have_lists);
-          if (lane == src) accumulate<CPLX>(acc, load_psi<CPLX>(psi, row), p0, hs);
-        }
+        push_singles<L>(q, qn, kind, y, row, 0u, flush);
       }
     }
+    if (qn) flush(qn);
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
@@ -714,7 +753,7 @@ eloc_eval_kernel(const u64 *__restrict__ bra, long long n, const double *__restr
       psi0_out[s] = p0.re;
     }
   }
-  __syncwarp();  // the next item reuses this warp's orbital lists
+  __syncwarp();  // the next item reuses this warp's orbital lists and queue
   if (list == nullptr) break;
   }
 }
@@ -745,10 +784,11 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
                       const HitRun *__restrict__ runs, const u32 *__restrict__ run_cnt, int run_stride, const u32 *__restrict__ hits,
                       const u32 *__restrict__ self_pos, const double *__restrict__ hii, double *__restrict__ eloc,
                       double *__restrict__ psi0_out, u32 *__restrict__ heavy_list, ElocCounters *ctr, ExcGeom g, int per_warp) {
-  __shared__ OrbLists s_lists[kEvalThreads / 32];
   __shared__ EvalTileSmem s_tile[kEvalThreads / 32];
+  __shared__ SingleQueue<L> s_queue[kEvalThreads / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   EvalTileSmem &T = s_tile[warp];
+  SingleQueue<L> &q = s_queue[warp];
   // per_warp: samples a warp takes (32; 16 or 8 when the call has too few samples to fill the GPU with 32 per warp -- the hit
   // lists are walked 32 hits at a time whatever the number of samples they belong to)
   const long long s0 = ((long long)blockIdx.x * (kEvalThreads / 32) + warp) * per_warp;
@@ -788,7 +828,37 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
   }
   __syncwarp();
   const int max_runs = __reduce_max_sync(0xffffffffu, heavy ? 0 : nruns);
-  int lists_owner = -1;
+  // lane i evaluates entry i; the products go into the samples' accumulators in queue order (lane l adds those of sample l:
+  // the entries of one sample need not be adjacent, so segment tails added in parallel would race); four terms in flight
+  u32 qn = 0;
+  auto flush = [&](u32 cnt) {
+    Cplx v = {0.0, 0.0};
+    u32 jq = 32;
+    if ((u32)lane < cnt) {
+      jq = q.j[lane];
+      Onv<L> xq, yq;
+#pragma unroll
+      for (int w = 0; w < L; ++w) {
+        xq.w[w] = T.x[jq][w];
+        yq.w[w] = q.y[lane][w];
+      }
+      const Cplx pq = {T.p0[jq][0], T.p0[jq][1]};
+      accumulate<CPLX>(v, load_psi<CPLX>(psi, q.row[lane]), pq, single_element<L, 4, double>(xq, yq, h1e, h2e, g.sorb));
+    }
+    Cplx a = {T.acc[lane][0], T.acc[lane][1]};
+    for (u32 i = 0; i < cnt; ++i) {
+      const u32 ji = __shfl_sync(0xffffffffu, jq, i);
+      const double vr = __shfl_sync(0xffffffffu, v.re, i);
+      const double vi = CPLX ? __shfl_sync(0xffffffffu, v.im, i) : 0.0;
+      if (ji == (u32)lane) {
+        a.re += vr;
+        if (CPLX) a.im += vi;
+      }
+    }
+    T.acc[lane][0] = a.re;
+    T.acc[lane][1] = a.im;
+    __syncwarp();
+  };
   for (int r = 0; r < max_runs; ++r) {
     HitRun mine = {0u, 0u};
     if (!heavy && r < nruns) mine = my_runs[r];
@@ -809,27 +879,7 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
       Cplx v = {0.0, 0.0};
       const Cplx pj = {T.p0[j][0], T.p0[j][1]};
       if (kind == 2) accumulate<CPLX>(v, load_psi<CPLX>(psi, row), pj, double_element<L, double>(xs, y, h2e));
-      // single excitations (rare): one at a time by the whole warp, terms gathered in parallel
-      u32 pend = __ballot_sync(0xffffffffu, kind == 1);
-      while (pend) {
-        const int src = __ffs(pend) - 1;
-        pend &= pend - 1u;
-        const int js = __shfl_sync(0xffffffffu, j, src);
-        Onv<L> xb, yb;
-#pragma unroll
-        for (int w = 0; w < L; ++w) {
-          xb.w[w] = T.x[js][w];
-          yb.w[w] = __shfl_sync(0xffffffffu, y.w[w], src);
-        }
-        if (lists_owner != js) {
-          __syncwarp();
-          build_lists<L>(xb, g.sorb, g.noA, g.noB, s_lists[warp], lane);
-          __syncwarp();
-          lists_owner = js;
-        }
-        const double hv = single_element_warp<L, double>(xb, yb, h1e, h2e, g.sorb, s_lists[warp].occ_order, s_lists[warp].n_occ);
-        if (lane == src) accumulate<CPLX>(v, load_psi<CPLX>(psi, row), pj, hv);
-      }
+      push_singles<L>(q, qn, kind, y, row, (u32)j, flush);
       // sum of v over the lanes of the same sample (adjacent), then the last lane of every sample adds it in
       const int jkey = e < total ? j : 32 + lane;  // idle lanes: segments of their own
 #pragma unroll
@@ -850,6 +900,7 @@ eloc_eval_tile_kernel(const u64 *__restrict__ bra, long long n, const double *__
       __syncwarp();
     }
   }
+  if (qn) flush(qn);
   __syncwarp();
   const Cplx acc = {T.acc[lane][0], T.acc[lane][1]};
   if (valid && !heavy) {

@@ -111,6 +111,50 @@ __device__ __forceinline__ T double_element(const Onv<L> &x, const Onv<L> &y, co
   return v;
 }
 
+// Single excitation x -> y evaluated by one lane: the excitation re-derived as in rederived_element, then exc_element's single
+// branch -- the same terms (two_body) added in the same order (occupied orbitals by word ascending, bits descending), so the
+// same value.  The terms are loaded AHEAD at a time before they are added, instead of one dependent load per addition (each
+// term in flight holds a register of the caller's budget).
+template <int L, int AHEAD, typename T>
+__device__ __forceinline__ T single_element(const Onv<L> &x, const Onv<L> &y, const T *__restrict__ h1e, const T *__restrict__ h2e,
+                                            int sorb) {
+  Onv<L> cre, ann;
+#pragma unroll
+  for (int i = 0; i < L; ++i) {
+    const u64 d = x.w[i] ^ y.w[i];
+    cre.w[i] = d & x.w[i];
+    ann.w[i] = d & y.w[i];
+  }
+  const u32 h = (u32)pop_highest<L>(cre), p = (u32)pop_highest<L>(ann);
+  T v = (T)0.0;
+  v += __ldg(h1e + (size_t)p * sorb + h);
+#pragma unroll
+  for (int i = 0; i < L; ++i) {
+    u64 rest = x.w[i];
+    while (rest) {
+      T t[AHEAD];
+      int n = 0;
+#pragma unroll
+      for (int u = 0; u < AHEAD; ++u) {
+        t[u] = (T)0.0;
+        if (rest) {
+          const int b = 63 - __clzll((long long)rest);
+          rest ^= 1ull << b;
+          const u32 k = (u32)(64 * i + b);
+          t[u] = two_body<T>(h2e, h, k, p, k);
+          n = u + 1;
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < AHEAD; ++u)
+        if (u < n) v += t[u];
+    }
+  }
+  const int sg = (count_below<L>(x, (int)h) ^ count_below<L>(x, (int)p) ^ (int)(h < p)) & 1;
+  v *= sg ? (T)-1.0 : (T)1.0;
+  return v;
+}
+
 // Single excitation x -> y evaluated by a whole warp (all lanes pass the same x, y): the two-electron terms
 // of cpp_src/cpu/hamiltonian.cpp:52-72 are gathered one per lane and then added in the reference's order
 // (occ_order: words ascending, bits descending) through shuffles -- the same additions in the same order as
