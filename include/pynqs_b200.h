@@ -214,6 +214,35 @@ int pynqs_rdm_scratch_bytes(int64_t N, int64_t nnz, int sorb, int64_t *bytes);
 int pynqs_rdm_offdiag(const int64_t *crow, const int64_t *col, const uint8_t *key, int64_t N, int64_t nnz, int sorb, const double *c,
                       int c_complex, void *scratch, int64_t scratch_bytes, double *dm1, double *dm2, void *stream);
 
+/* Additive op: the Epstein-Nesbet second-order correction of real states C over the sorted key table (N unique keys of one
+ * (noA, noB) sector, (sorb - 1) / 64 + 1 words; group_ws built by pynqs_group_build for it):
+ *   acc[r] += sum over the externals a of (sum over i of <key_i|H|a> C[i, r])^2 / (E[r] - <a|H|a>)
+ * where the externals are the distinct single and double excitations of the table rows (the rows of get_comb_tensor) that
+ * are not in the table, <key_i|H|a> has the bits of pynqs_comb_hij_fused and <a|H|a> those of pynqs_hij(a, a).  Not
+ * normalised: the caller divides by sum_i C[i, r]^2.  The externals are split into 2^log2_parts partitions by a hash of the
+ * determinant; one pass handles partition `part` completely, in four calls on one scratch buffer:
+ *   pynqs_pt2_count : offsets int64[N + 1] = exclusive prefix of the rows' kept (row, external) pairs, offsets[N] = pairs;
+ *   pynqs_pt2_emit  : per pair, the external and (<key_i|H|a>, i), rows ascending, each row's excitations ascending;
+ *   pynqs_pt2_sort  : the pairs sorted by external, stable (pynqs_sort_table's sort);
+ *   pynqs_pt2_reduce: acc[r] += the pass's sum (r < k <= 8; C double[N, k] with row stride ldc, E double[k]; wider blocks in
+ *                     column slices), externals[0] += the pass's externals (externals may be NULL).
+ * scratch: pynqs_pt2_scratch_bytes(N, pairs, sorb) bytes -- size it for pairs = 0 for the count call and for the pass's
+ * pairs (offsets[N], read by the caller) for the other three.  Deterministic (no float atomics; each numerator summed in
+ * ascending (row, excitation) order, the externals' terms in an order fixed by the sorted pairs and a fixed grid): two calls
+ * give identical bits; adding the passes' sums in pass order makes the whole sum deterministic for a given log2_parts.  No
+ * host synchronisation.  PYNQS_EVALUE, before anything touches the device, for an odd sorb or one outside
+ * (0, PYNQS_MAX_SORB], N outside (0, 2^31), pairs outside [0, 2^31), a bad sector, part outside [0, 2^log2_parts),
+ * log2_parts outside [0, 31], nele outside [0, sorb], k outside [1, 8], ldc < k, or a NULL pointer other than externals.
+ * The table must not hold duplicate keys (the caller's to refuse).  pairs == 0 makes emit, sort and reduce do nothing. */
+int pynqs_pt2_scratch_bytes(int64_t N, int64_t pairs, int sorb, int64_t *bytes);
+int pynqs_pt2_count(const uint8_t *key, int64_t N, int sorb, int noA, int noB, const void *group_ws, int part, int log2_parts, void *scratch,
+                    int64_t scratch_bytes, int64_t *offsets, void *stream);
+int pynqs_pt2_emit(const uint8_t *key, int64_t N, const double *h1e, const void *prep_ws, int sorb, int noA, int noB, const void *group_ws,
+                   int part, int log2_parts, const int64_t *offsets, int64_t pairs, void *scratch, int64_t scratch_bytes, void *stream);
+int pynqs_pt2_sort(int64_t N, int64_t pairs, int sorb, void *scratch, int64_t scratch_bytes, void *stream);
+int pynqs_pt2_reduce(int64_t N, int64_t pairs, const double *h1e, const double *h2e, int sorb, int nele, const double *C, int64_t ldc, int k,
+                     const double *E, void *scratch, int64_t scratch_bytes, double *acc, int64_t *externals, void *stream);
+
 /* ---- REDUCE method (vmc/energy/eloc.py:257-297, additive) -----------------------------------------
  * The reference materialises comb [n, M, 8L] and Hmat [n, M] and keeps torch.where(|Hmat| >= eps).  These
  * entry points return the kept rows only, in the same (ascending flat index s * M + m) order:

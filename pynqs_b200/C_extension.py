@@ -797,6 +797,94 @@ def rdm_offdiag(crow: Tensor, col: Tensor, bra_key: Tensor, c: Tensor, sorb: int
     return dm1, dm2
 
 
+_PT2_MAX_PAIRS = (1 << 31) - 1  # pairs of one pass: the table sort's limit
+
+
+def pt2_log2_parts(upper_pairs: int, max_bytes: int, pass_bytes) -> int:
+    """log2 of the smallest power of two P for which a pass of ceil(upper_pairs / P) pairs needs at most max_bytes of scratch
+    (pass_bytes(pairs) -> bytes) and stays below 2^31 pairs.  ValueError when no P does."""
+    lg = 0
+    while True:
+        pairs = -(-upper_pairs // (1 << lg))
+        if pairs <= _PT2_MAX_PAIRS and pass_bytes(pairs) <= max_bytes:
+            return lg
+        if pairs <= 1 or lg >= 31:
+            raise ValueError(f"max_bytes = {max_bytes} cannot hold a pass of the PT2 sum ({pass_bytes(1)} bytes at one pair)")
+        lg += 1
+
+
+def pt2_sums(bra_key: Tensor, C: Tensor, E: Tensor, h1e: Tensor, h2e: Tensor, sorb: int, nele: int, noA: int, noB: int,
+             group_index: GroupIndex | None = None, max_bytes: int = 16 << 30) -> Tuple[Tensor, dict]:
+    """The unnormalised Epstein-Nesbet sums of the columns of C over the sorted unique table bra_key (pynqs_pt2_*):
+    acc[r] = sum over the externals a of (sum_i <key_i|H|a> C[i, r])^2 / (E[r] - <a|H|a>), float64 [k].  C: float64 [N, k]
+    (any k: column slices of 8), E: float64 [k].  The externals are split into P = 2^log2 partitions, P the smallest power
+    of two for which the scratch of a pass of N * nsd / P pairs fits in max_bytes (pt2_log2_parts); a partition whose exact
+    count does not fit doubles P and restarts.  The passes' sums are added in pass order.  Returns (acc, info) with info["externals"],
+    info["pairs"] and info["passes"].  Deterministic for a given P; one host synchronisation per pass."""
+    dev = _need_cuda(bra_key, C, E, h1e, h2e)
+    for t, nm in ((bra_key, "bra_key"), (h1e, "h1e"), (h2e, "h2e")):
+        _contig(t, nm)
+    if bra_key.dim() != 2 or C.dim() != 2 or C.size(0) != bra_key.size(0) or E.shape != (C.size(1),):
+        raise ValueError("bra_key must be [N, 8L], C [N, k] and E [k]")
+    if C.dtype != torch.float64 or E.dtype != torch.float64 or h1e.dtype != torch.float64 or h2e.dtype != torch.float64:
+        raise ValueError("pt2_sums needs float64 C, E and integrals")
+    _check_width(bra_key, sorb, "bra_key")
+    _check_integrals(h1e, h2e, sorb)
+    nsd = get_Num_SinglesDoubles(sorb, noA, noB)
+    N, kk = bra_key.size(0), C.size(1)
+    if N == 0:
+        raise ValueError("the table is empty")
+    if group_index is None:
+        group_index = _cached_group(bra_key)
+    if group_index.N != N or group_index.L != bra_key.size(1) // 8 or group_index.key_ptr != bra_key.data_ptr():
+        raise ValueError("group_index was built for another key table")
+    C = C.contiguous()
+    E = E.contiguous()
+    lib = _lib.load()
+
+    def scratch_bytes(pairs: int) -> int:
+        nb = _lib.ctypes.c_int64()
+        _lib.check(lib.pynqs_pt2_scratch_bytes(i64(N), i64(pairs), int(sorb), _lib.ctypes.byref(nb)))
+        return nb.value
+
+    prep = _cached_prep(h2e, sorb)
+    key = (vp(bra_key.data_ptr()), i64(N))
+    lg = pt2_log2_parts(N * nsd, max_bytes, scratch_bytes)
+    with torch.cuda.device(dev):
+        offsets = torch.empty(N + 1, dtype=torch.int64, device=dev)
+        count_scratch = torch.empty(scratch_bytes(0), dtype=torch.uint8, device=dev)
+        while True:
+            acc = torch.zeros(kk, dtype=torch.float64, device=dev)
+            externals = torch.zeros(1, dtype=torch.int64, device=dev)
+            pairs_total, restart = 0, False
+            for part in range(1 << lg):
+                sel = (vp(group_index.workspace.data_ptr()), int(part), int(lg))
+                _lib.check(lib.pynqs_pt2_count(*key, int(sorb), int(noA), int(noB), *sel, vp(count_scratch.data_ptr()),
+                                               i64(count_scratch.numel()), vp(offsets.data_ptr()), _stream(dev)))
+                pairs = int(offsets[N].item())
+                if pairs > _PT2_MAX_PAIRS or scratch_bytes(pairs) > max_bytes:  # a partition larger than planned
+                    restart = True
+                    break
+                if pairs == 0:
+                    continue
+                pairs_total += pairs
+                scratch = torch.empty(scratch_bytes(pairs), dtype=torch.uint8, device=dev)
+                sc = (vp(scratch.data_ptr()), i64(scratch.numel()))
+                _lib.check(lib.pynqs_pt2_emit(*key, vp(h1e.data_ptr()), vp(prep.workspace.data_ptr()), int(sorb), int(noA), int(noB), *sel,
+                                              vp(offsets.data_ptr()), i64(pairs), *sc, _stream(dev)))
+                _lib.check(lib.pynqs_pt2_sort(i64(N), i64(pairs), int(sorb), *sc, _stream(dev)))
+                for c0 in range(0, kk, 8):
+                    k = min(8, kk - c0)
+                    _lib.check(lib.pynqs_pt2_reduce(i64(N), i64(pairs), vp(h1e.data_ptr()), vp(h2e.data_ptr()), int(sorb), int(nele),
+                                                    vp(C.data_ptr() + 8 * c0), i64(kk), int(k), vp(E.data_ptr() + 8 * c0), *sc,
+                                                    vp(acc.data_ptr() + 8 * c0), vp(externals.data_ptr() if c0 == 0 else None),
+                                                    _stream(dev)))
+                del scratch
+            if not restart:
+                return acc, {"externals": int(externals.item()), "pairs": pairs_total, "passes": 1 << lg}
+            lg += 1
+
+
 def lookup_compact(idx_array: Tensor, mask: Tensor, wf_value: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
     """(positions with mask set, positions without, wf_value[idx_array[mask]]) -- the index glue of
     WavefunctionLUT.lookup (utils/public_function.py:825-838: arange, two boolean-mask selections, masked_select, gather)

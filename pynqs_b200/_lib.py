@@ -17,6 +17,7 @@ SYMBOLS = [
     "pynqs_group_bytes", "pynqs_group_build", "pynqs_group_layout", "pynqs_eloc_scratch_bytes", "pynqs_eloc_sample_space",
     "pynqs_hamiltonian_scratch_bytes", "pynqs_hamiltonian_count", "pynqs_hamiltonian_emit", "pynqs_csr_spmm",
     "pynqs_spin_square_apply", "pynqs_rdm_scratch_bytes", "pynqs_rdm_offdiag",
+    "pynqs_pt2_scratch_bytes", "pynqs_pt2_count", "pynqs_pt2_emit", "pynqs_pt2_sort", "pynqs_pt2_reduce",
     "pynqs_reduce_scratch_bytes", "pynqs_reduce_count", "pynqs_reduce_emit", "pynqs_reduce_eloc",
     "pynqs_reduce_sample_scratch_bytes", "pynqs_reduce_sample_count", "pynqs_reduce_sample_emit",
     "pynqs_compact_scratch_bytes", "pynqs_lookup_count", "pynqs_lookup_emit", "pynqs_unique_count", "pynqs_unique_emit",

@@ -9,8 +9,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libpynqs_b200.so")
-SOURCES = ["abi.cu", "enumerate.cu", "hij.cu", "lut.cu", "eloc_scan.cu", "eloc_block.cu", "hamiltonian.cu", "spmm.cu", "spin.cu", "rdm.cu", "gindex.cu", "convert.cu", "reduce_sample.cu", "compact.cu", "peer.cu", "prepare.cu", "table.cu"]
-HEADERS = ["common.cuh", "lut.cuh", "tables.cuh", "prepare.cuh", "gindex.cuh", "eloc.cuh", "rederive.cuh", os.path.join("..", "..", "include", "pynqs_b200.h")]
+SOURCES = ["abi.cu", "enumerate.cu", "hij.cu", "lut.cu", "eloc_scan.cu", "eloc_block.cu", "hamiltonian.cu", "spmm.cu", "spin.cu", "rdm.cu", "pt2.cu", "gindex.cu", "convert.cu", "reduce_sample.cu", "compact.cu", "peer.cu", "prepare.cu", "table.cu"]
+HEADERS = ["common.cuh", "lut.cuh", "tables.cuh", "prepare.cuh", "gindex.cuh", "eloc.cuh", "rederive.cuh", "enum_rows.cuh", os.path.join("..", "..", "include", "pynqs_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -88,6 +88,12 @@ int launch_spin_square(const u64 *, long long, int, const u64 *, long long, cons
 long long rdm_scratch_bytes(long long);
 int launch_rdm(const long long *, const long long *, const u64 *, long long, long long, int, const double *, int, void *, long long, double *,
                double *, cudaStream_t);
+long long pt2_scratch_bytes(long long, long long, int);
+int launch_pt2_rows(const u64 *, long long, const double *, const void *, const void *, int, int, long long *, long long, void *, long long,
+                    const ExcGeom &, int, cudaStream_t);
+int launch_pt2_sort(long long, long long, int, void *, long long, cudaStream_t);
+int launch_pt2_reduce(long long, long long, const double *, const double *, int, int, const double *, long long, int, const double *, void *,
+                      long long, double *, long long *, cudaStream_t);
 
 static int check_geometry(int sorb, int nele, int noA, int noB) {
   if (sorb <= 0 || sorb > PYNQS_MAX_SORB) {
@@ -528,6 +534,86 @@ int pynqs_rdm_offdiag(const int64_t *crow, const int64_t *col, const uint8_t *ke
   if (N == 0 || nnz == 0) return 0;
   return launch_rdm(reinterpret_cast<const long long *>(crow), reinterpret_cast<const long long *>(col), reinterpret_cast<const u64 *>(key), N,
                     nnz, sorb, c, c_complex, scratch, scratch_bytes, dm1, dm2, st);
+}
+
+static int pt2_check(const char *what, int64_t N, int64_t pairs, int sorb) {
+  if (sorb <= 0 || sorb > PYNQS_MAX_SORB || (sorb & 1)) {
+    set_error("%s: sorb = %d must be even and in (0, %d]", what, sorb, PYNQS_MAX_SORB);
+    return PYNQS_EVALUE;
+  }
+  if (N <= 0 || N >= (1LL << 31) || pairs < 0 || pairs >= (1LL << 31)) {
+    set_error("%s: bad N = %lld or pairs = %lld (0 < N < 2^31, 0 <= pairs < 2^31)", what, (long long)N, (long long)pairs);
+    return PYNQS_EVALUE;
+  }
+  return 0;
+}
+
+static int pt2_rows_common(const char *what, const uint8_t *key, int64_t N, const double *h1e, const void *prep_ws, int sorb, int noA, int noB,
+                           const void *group_ws, int part, int log2_parts, int64_t *offsets, int64_t pairs, void *scratch,
+                           int64_t scratch_bytes, int emit, void *stream) {
+  if (int rc = check_geometry(sorb, noA + noB, noA, noB)) return rc;
+  long long nsd;
+  if (int rc = num_sd_checked(sorb, noA, noB, &nsd)) return rc;
+  if (int rc = pt2_check(what, N, pairs, sorb)) return rc;
+  if (log2_parts < 0 || log2_parts > 31 || part < 0 || (long long)part >= (1LL << log2_parts)) {
+    set_error("%s: bad part = %d of 2^%d partitions", what, part, log2_parts);
+    return PYNQS_EVALUE;
+  }
+  if (key == nullptr || group_ws == nullptr || scratch == nullptr || offsets == nullptr || (emit && (h1e == nullptr || prep_ws == nullptr))) {
+    set_error("%s: null pointer (key / group_ws / scratch / offsets, h1e / prep_ws for the emit call)", what);
+    return PYNQS_EVALUE;
+  }
+  if (emit && pairs == 0) return 0;
+  return launch_pt2_rows(reinterpret_cast<const u64 *>(key), N, h1e, prep_ws, group_ws, part, log2_parts, reinterpret_cast<long long *>(offsets),
+                         pairs, scratch, scratch_bytes, make_geom(sorb, noA + noB, noA, noB), emit, (cudaStream_t)stream);
+}
+
+int pynqs_pt2_scratch_bytes(int64_t N, int64_t pairs, int sorb, int64_t *bytes) {
+  if (int rc = pt2_check("pt2_scratch_bytes", N, pairs, sorb)) return rc;
+  if (bytes == nullptr) {
+    set_error("pt2_scratch_bytes: null bytes");
+    return PYNQS_EVALUE;
+  }
+  *bytes = pt2_scratch_bytes(N, pairs, (sorb - 1) / 64 + 1);
+  return 0;
+}
+
+int pynqs_pt2_count(const uint8_t *key, int64_t N, int sorb, int noA, int noB, const void *group_ws, int part, int log2_parts, void *scratch,
+                    int64_t scratch_bytes, int64_t *offsets, void *stream) {
+  return pt2_rows_common("pt2_count", key, N, nullptr, nullptr, sorb, noA, noB, group_ws, part, log2_parts, offsets, 0, scratch, scratch_bytes,
+                         0, stream);
+}
+
+int pynqs_pt2_emit(const uint8_t *key, int64_t N, const double *h1e, const void *prep_ws, int sorb, int noA, int noB, const void *group_ws,
+                   int part, int log2_parts, const int64_t *offsets, int64_t pairs, void *scratch, int64_t scratch_bytes, void *stream) {
+  return pt2_rows_common("pt2_emit", key, N, h1e, prep_ws, sorb, noA, noB, group_ws, part, log2_parts, const_cast<int64_t *>(offsets), pairs,
+                         scratch, scratch_bytes, 1, stream);
+}
+
+int pynqs_pt2_sort(int64_t N, int64_t pairs, int sorb, void *scratch, int64_t scratch_bytes, void *stream) {
+  if (int rc = pt2_check("pt2_sort", N, pairs, sorb)) return rc;
+  if (scratch == nullptr) {
+    set_error("pt2_sort: null scratch");
+    return PYNQS_EVALUE;
+  }
+  if (pairs == 0) return 0;
+  return launch_pt2_sort(N, pairs, sorb, scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+int pynqs_pt2_reduce(int64_t N, int64_t pairs, const double *h1e, const double *h2e, int sorb, int nele, const double *C, int64_t ldc, int k,
+                     const double *E, void *scratch, int64_t scratch_bytes, double *acc, int64_t *externals, void *stream) {
+  if (int rc = pt2_check("pt2_reduce", N, pairs, sorb)) return rc;
+  if (nele < 0 || nele > sorb || k < 1 || k > 8 || ldc < k) {
+    set_error("pt2_reduce: bad nele = %d, k = %d or ldc = %lld (k in [1, 8], ldc >= k)", nele, k, (long long)ldc);
+    return PYNQS_EVALUE;
+  }
+  if (h1e == nullptr || h2e == nullptr || C == nullptr || E == nullptr || scratch == nullptr || acc == nullptr) {
+    set_error("pt2_reduce: null pointer (h1e / h2e / C / E / scratch / acc)");
+    return PYNQS_EVALUE;
+  }
+  if (pairs == 0) return 0;
+  return launch_pt2_reduce(N, pairs, h1e, h2e, sorb, nele, C, ldc, k, E, scratch, scratch_bytes, acc, reinterpret_cast<long long *>(externals),
+                           (cudaStream_t)stream);
 }
 
 int64_t pynqs_reduce_scratch_bytes(int64_t n) { return reduce_scratch_bytes(n); }

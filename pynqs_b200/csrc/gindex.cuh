@@ -25,6 +25,7 @@
 // still separates them, so collisions cost a little work and never change a result.
 #pragma once
 #include "common.cuh"
+#include "lut.cuh"
 
 namespace pynqs {
 
@@ -107,6 +108,15 @@ __device__ __forceinline__ u32 bucket_search(const u64 *__restrict__ keys, u32 l
     else hi = mid;
   }
   return 0xffffffffu;
+}
+
+// table row of y, or -1: the beta-grouped copy, or the classic binary search over a table with duplicate keys
+template <int L>
+__device__ __forceinline__ long long spin_find(const u64 *__restrict__ key, long long N, const GroupView &gv, bool dup, const Onv<L> &y) {
+  if (dup) return classic_search<L>(key, N, y);
+  const u32 b = group_bucket<L>(y, 0, gv.shift);
+  const u32 pos = bucket_search<L>(gv.keys[0], __ldg(gv.start[0] + b), __ldg(gv.start[0] + b + 1), y);
+  return pos == 0xffffffffu ? -1 : (long long)__ldg(gv.rows[0] + pos);
 }
 
 // host side (gindex.cu)

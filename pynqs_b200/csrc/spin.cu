@@ -25,15 +25,6 @@ namespace pynqs {
 constexpr int kSpinThreads = 128;  // 8 CTAs per SM at least: the 64-register cap leaves every (L, K) variant free of spills
 constexpr long long kSpinBlocksCap = 148LL * 16 * 8;  // a grid-stride loop past ~2.4 * 10^6 rows
 
-// table row of y, or -1
-template <int L>
-__device__ __forceinline__ long long spin_find(const u64 *__restrict__ key, long long N, const GroupView &gv, bool dup, const Onv<L> &y) {
-  if (dup) return classic_search<L>(key, N, y);
-  const u32 b = group_bucket<L>(y, 0, gv.shift);
-  const u32 pos = bucket_search<L>(gv.keys[0], __ldg(gv.start[0] + b), __ldg(gv.start[0] + b + 1), y);
-  return pos == 0xffffffffu ? -1 : (long long)__ldg(gv.rows[0] + pos);
-}
-
 template <int L, int K>
 __global__ void __launch_bounds__(kSpinThreads, 8)
 spin_square_kernel(const u64 *__restrict__ bra, long long n, const u64 *__restrict__ key, long long N, GroupView gv,

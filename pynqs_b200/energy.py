@@ -124,6 +124,46 @@ def sample_space_ground_state(WF_LUT: WavefunctionLUT, h1e: Tensor, h2e: Tensor,
     return (C * h_apply(C)).sum(0) / norm, C, info
 
 
+def sample_space_pt2(WF_LUT: WavefunctionLUT, C: Tensor, energies: Tensor, h1e: Tensor, h2e: Tensor, sorb: int, nele: int, noa: int,
+                     nob: int, *, max_bytes: int = 16 << 30) -> Tuple[Tensor, dict]:
+    """The Epstein-Nesbet second-order correction of sample-space states, what selected CI (CIPSI, HCI) reports next to the
+    variational energy as E_var + E_PT2:
+        E_PT2[r] = (1 / sum_i C[i, r]^2) sum over a in X of (sum_i <key_i|H|a> C[i, r])^2 / (E[r] - <a|H|a>)
+    with X the externals -- the distinct single and double excitations of the table's determinants (WF_LUT.bra_key, one
+    (noa, nob) sector, no duplicates) that are not in the table.  <key_i|H|a> has the bits of get_comb_hij_fused, <a|H|a>
+    those of get_hij_torch(a, a); both are electronic, like the energies of sample_space_ground_state, so
+    `e, C, _ = sample_space_ground_state(...)` passes straight through.  A table that is the whole sector gives 0.
+
+    C: float64 [N] or [N, k] (columns = states, rows in the order of WF_LUT.bra_key); energies: [k].  Returns (e_pt2 float64
+    [k], info) with info["externals"] = |X|, info["pairs"] = the (row, external) pairs summed, info["passes"].  The externals
+    are handled in passes of a hash partition each, as many as it takes to keep a pass's scratch within max_bytes (a memory
+    limit; it changes the result only by rounding).  Deterministic: two calls with the same inputs and max_bytes give
+    identical bits.  ValueError for a C of the wrong shape or dtype, energies of the wrong length, a zero column, a table
+    with duplicate keys, non-float64 integrals or an empty table."""
+    keys = WF_LUT.bra_key
+    N = keys.size(0)
+    if N == 0:
+        raise ValueError("the table is empty")
+    if C.dtype != torch.float64 or C.dim() not in (1, 2) or C.size(0) != N:
+        raise ValueError(f"C must be float64 [N] or [N, k] with N = {N}, got {C.dtype} {tuple(C.shape)}")
+    C2 = C.unsqueeze(1) if C.dim() == 1 else C
+    k = C2.size(1)
+    energies = torch.as_tensor(energies, dtype=torch.float64, device=keys.device).reshape(-1)
+    if energies.numel() != k or k == 0:
+        raise ValueError(f"energies must hold one value per column of C ({k}), got {energies.numel()}")
+    if h1e.dtype != torch.float64 or h2e.dtype != torch.float64:
+        raise ValueError("sample_space_pt2 needs float64 integrals")
+    norm = (C2 * C2).sum(0)
+    dup = (keys[1:] == keys[:-1]).all(1).any() if N > 1 else torch.zeros((), dtype=torch.bool, device=keys.device)
+    zero, has_dup = torch.stack([(norm == 0).any(), dup]).tolist()
+    if zero:
+        raise ValueError("C has a column with sum c^2 = 0")
+    if has_dup:
+        raise ValueError("the table has duplicate keys")
+    acc, info = ops.pt2_sums(keys, C2, energies, h1e, h2e, sorb, nele, noa, nob, WF_LUT.group_index, max_bytes=max_bytes)
+    return acc / norm, info
+
+
 def _spin_diagonal(x: Tensor) -> Tensor:
     """<x|S^2|x> = |B| + Sz (Sz + 1) of every ONV row of x (uint8 [n, 8L]), float64 [n]: B = the beta-only orbitals,
     Sz = (n_alpha - n_beta) / 2 (alpha on the even bits, beta on the odd ones)."""
